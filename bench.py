@@ -1,10 +1,14 @@
 #!/usr/bin/env python
 """bench.py — the headline measurement of the SpMM hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--k 64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--k 64] [--dump-outputs DIR]
 
 One "step" = one pass C = A*B of the cop20k_A-shaped k=64 SpMM (BASELINE.json configs[1], the
-configuration the north_star target is quoted on) over one resident operand set. With N > 1 (one
+configuration the north_star target is quoted on) over one resident operand set. A and B are seeded,
+so the same arguments give the same inputs in every run; --dump-outputs DIR writes the C of the last
+timed step as DIR/C.npy (float64; DIR/C_rank<r>.npy per rank at N > 1), a fixed sample of its rows
+when it would exceed 64 MB, so that two builds can be compared output for output. It applies to the
+GPU path only: --impl reference times the CPU code without keeping its result. With N > 1 (one
 process per GPU under torchrun) every rank owns one cop20k_A-shaped diagonal block of a
 (N*121,192)-row block-diagonal matrix — the row-wise partition (RowWise.cpp:26-29) of a matrix whose
 blocks read only their own rows of B, so no byte has to cross a link (weak scaling, no collective
@@ -38,11 +42,23 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark leaves the tree it runs from as it found it: build() never imports oracle/pyoracle.py, so without this
+# the first run would add oracle/__pycache__/ to a tree that has just been built
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 
 N_ROWS, NNZ = 121_192, 2_624_331
 OPERAND_SETS = 4  # rotating resident copies of (A, B, C): 4 x ~175 MB >> 126 MB L2
+DUMP_BYTES = 63_000_000  # array bytes --dump-outputs writes over every rank: under 64 MB with the .npy headers
+
+
+def dump_output(path: str, C: np.ndarray, budget: int) -> None:
+    """C as .npy; a fixed, seeded sample of its rows (in row order) when it is larger than `budget` bytes."""
+    if C.nbytes > budget:
+        keep = budget // (C.shape[1] * C.itemsize)
+        C = C[np.sort(np.random.default_rng(0).choice(C.shape[0], keep, replace=False))]
+    np.save(path, C)
 
 
 def algorithmic_bytes(n_rows: int, nnz: int, k: int) -> int:
@@ -233,7 +249,12 @@ def main():
     ap.add_argument("--kernel", default="auto")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip configs_1gpu / north_star_scaling (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the C of the last timed step to DIR as .npy (--impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the output of the GPU path (--impl ours)")
     k = args.k
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -315,7 +336,9 @@ def main():
         A = first if s == 0 else spmm.DeviceCSR.from_host(host, local_rank)
         if args.kernel in ("auto", "tiled"):
             A.build_tiles(-1, 0, k)  # what AUTO does by itself on its first multiply; done here so it is outside any timing
-        Bd = torch.randint(1, 101, (n, k), device=dev).double()
+        gen_b = torch.Generator(device=dev)
+        gen_b.manual_seed(OPERAND_SETS * rank + s)
+        Bd = torch.randint(1, 101, (n, k), device=dev, generator=gen_b).double()
         Cd = torch.empty((n, k), dtype=torch.float64, device=dev)
         sets.append((A, Bd, Cd))
     tiles = sets[0][0].tile_info()
@@ -340,6 +363,10 @@ def main():
     barrier()
     wall = time.perf_counter() - t_wall
     clocks = sampler.stop()
+    if args.dump_outputs:  # read back now: the L2-warm pass below writes the C of operand set 0 again
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dump_output(os.path.join(args.dump_outputs, "C.npy" if world == 1 else f"C_rank{rank}.npy"),
+                    sets[(args.steps - 1) % OPERAND_SETS][2].cpu().numpy(), DUMP_BYTES // world)
     ms_per_step = tmax(ev0.elapsed_time(ev1)) / args.steps
     # beside it (SURVEY 8d: "both L2-warm and L2-flushed"): the same launches on ONE operand set, whatever fits stays in L2
     w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

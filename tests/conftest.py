@@ -24,7 +24,7 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def reference():
-    """The reference's own code compiled into oracle/_ref; present in the build container and, prebuilt, on the GPU box."""
+    """The reference's own code compiled into oracle/_ref by oracle/Makefile; only where its sources were given (REF=<dir>)."""
     import pyoracle
     if not pyoracle.Reference.available():
         pytest.skip("oracle/_ref not built (needs /root/reference at build time)")

@@ -105,11 +105,15 @@ def test_loader_against_compiled_reference_on_generated_file(oracle, reference, 
     assert a[2][-1] == 60001
 
 
-def test_are_equal_and_serialize(oracle, reference):
+def test_are_equal_and_serialize(oracle):
+    """areMatricesEqual's verdicts on either side of its bound; the compiled reference, where oracle/_ref is built, gives the same."""
+    import pyoracle
+    checkers = [oracle] + ([pyoracle.Reference("exact")] if pyoracle.Reference.available() else [])
     a = np.arange(12, dtype=np.float64).reshape(4, 3)
     b = a.copy()
     b[2, 1] += 5e-7
-    assert oracle.are_equal(a, b, 1e-6) and reference.are_equal(a, b, 1e-6)
+    assert all(x.are_equal(a, b, 1e-6) for x in checkers)
     b[2, 1] += 1e-6
-    assert not oracle.are_equal(a, b, 1e-6) and not reference.are_equal(a, b, 1e-6)
-    assert reference.serialize_is_rowmajor(a, 4, 3)
+    assert not any(x.are_equal(a, b, 1e-6) for x in checkers)
+    if len(checkers) > 1:
+        assert checkers[1].serialize_is_rowmajor(a, 4, 3)
