@@ -91,7 +91,21 @@ int spmm_csr_from_matrix_market(int device, const char *path, spmm_csr_t *out);
 
 int spmm_csr_destroy(spmm_csr_t A);
 int spmm_csr_info(spmm_csr_t A, int *n_rows, int *n_cols, long long *nnz, int *device);
+/* Writing through the returned value pointer requires spmm_csr_update_values_device(A, that pointer, stream) before the
+ * next multiply: without it the tiled kernel uses the old values (its layout holds a copy of them). */
 int spmm_csr_device_ptrs(spmm_csr_t A, const int **d_rowptr, const int **d_colidx, const double **d_vals);
+/* New values for the same pattern: vals[nnz] in the handle's CSR order. The schedule, the CTA cuts and the tile
+ * layout are kept; the values inside the tile layout are refreshed. Bits are copied (-0.0, NaN payloads survive).
+ * Whether the pattern is the same is not checked. nnz == 0: no-op; a NULL pointer otherwise: SPMM_ERR_INVALID.
+ * _device: enqueued on `stream`, returns without waiting. d_vals may be A's own value array (the pointer from
+ * spmm_csr_device_ptrs, or the caller's array behind a borrowed handle) after it was edited in place: then only the
+ * layout is refreshed. A borrowed handle (spmm_csr_create_device with copy=0) accepts no other pointer: the library
+ * never writes into memory lent to it as const. Multiplies enqueued later on other streams, the host-buffer forms
+ * included, must be ordered after `stream` by the caller; so must the update after earlier multiplies on other streams.
+ * _host: through the handle's pinned staging and host threads, on the handle's own stream (one host-buffer call per
+ * handle at a time); returns when the update is done, so `vals` may be reused. Not for borrowed handles. */
+int spmm_csr_update_values_device(spmm_csr_t A, const double *d_vals, void *stream);
+int spmm_csr_update_values_host(spmm_csr_t A, const double *vals);
 /* Copy the device CSR back (rowptr n_rows+1, colidx nnz, vals nnz) for memcmp-style checks. */
 int spmm_csr_download(spmm_csr_t A, int *rowptr, int *colidx, double *vals);
 /* Row-length schedule: bins[0..7] = rows with length 0, 1-2, 3-4, 5-8, 9-16, 17-32, 33-256, >256. */

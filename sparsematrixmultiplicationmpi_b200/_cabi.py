@@ -52,6 +52,8 @@ PROTOTYPES = {
     "spmm_csr_destroy": (_i, [_p]),
     "spmm_csr_info": (_i, [_p, _pi, _pi, _pll, _pi]),
     "spmm_csr_device_ptrs": (_i, [_p, C.POINTER(_p), C.POINTER(_p), C.POINTER(_p)]),
+    "spmm_csr_update_values_device": (_i, [_p, _p, _p]),
+    "spmm_csr_update_values_host": (_i, [_p, _p]),
     "spmm_csr_download": (_i, [_p, _p, _p, _p]),
     "spmm_csr_schedule": (_i, [_p, _pll, _pi, _pd, _pi]),
     "spmm_csr_column_block": (_i, [_p, _i, _i, C.POINTER(_p)]),

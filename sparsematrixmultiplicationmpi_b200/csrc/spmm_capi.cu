@@ -402,6 +402,18 @@ int spmm_csr_device_ptrs(spmm_csr_t A, const int **d_rowptr, const int **d_colid
     return SPMM_OK;
 }
 
+int spmm_csr_update_values_device(spmm_csr_t A, const double *d_vals, void *stream)
+{
+    SPMM_REQUIRE(A != nullptr, "handle is NULL");
+    if (A->nnz == 0)
+        return SPMM_OK;
+    SPMM_REQUIRE(d_vals != nullptr, "d_vals is NULL");
+    SPMM_REQUIRE(A->owns || d_vals == A->d_vals,
+                 "a borrowed handle reads the caller's value array: edit that array and pass it, the library does not write into it");
+    SPMM_CUDA(cudaSetDevice(A->device));
+    return update_values(A, d_vals, (cudaStream_t)stream);
+}
+
 int spmm_csr_download(spmm_csr_t A, int *rowptr, int *colidx, double *vals)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");

@@ -753,6 +753,31 @@ int spmm_fetch_c_rows(spmm_csr_t A, const double *d_C, int n_rows, int k, double
     return spmm_fetch_c_sink(A, d_C, n_rows, k, copy_sink, &cs);
 }
 
+namespace
+{
+// spmm_upload_dense without the lock and the final wait (the caller holds A->host_mu); a staged upload has finished when it
+// returns (its ring goes back to the free list)
+int upload_block(spmm_csr_t A, const double *src, long long n_rows, int k, double *d_dst, cudaStream_t stream)
+{
+    if (is_pinned(src))
+    {
+        SPMM_CUDA(cudaMemcpyAsync(d_dst, src, sizeof(double) * (size_t)n_rows * (size_t)k, cudaMemcpyHostToDevice, stream));
+        return SPMM_OK;
+    }
+    RingLease lease;
+    int rc = borrow_ring(A->device, ring_want(n_rows, k), &lease.r);
+    HostRows b;
+    b.flat = src;
+    b.ld = k;
+    if (!rc)
+        rc = staged_upload(*lease.r, A->device, b, d_dst, 0, (int)n_rows, k, stream);
+    if (rc)
+        return rc;
+    SPMM_CUDA(cudaStreamSynchronize(stream)); // before the ring goes back to the free list
+    return SPMM_OK;
+}
+} // namespace
+
 int spmm_upload_dense(spmm_csr_t A, const double *src, long long n_rows, int k, double *d_dst, void *stream)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
@@ -762,24 +787,37 @@ int spmm_upload_dense(spmm_csr_t A, const double *src, long long n_rows, int k, 
     SPMM_REQUIRE(src != nullptr && d_dst != nullptr, "src / d_dst is NULL");
     SPMM_CUDA(cudaSetDevice(A->device));
     std::lock_guard<std::mutex> guard(A->host_mu);
-    if (is_pinned(src))
-        SPMM_CUDA(cudaMemcpyAsync(d_dst, src, sizeof(double) * (size_t)n_rows * (size_t)k, cudaMemcpyHostToDevice, (cudaStream_t)stream));
-    else
-    {
-        RingLease lease;
-        int rc = borrow_ring(A->device, ring_want(n_rows, k), &lease.r);
-        HostRows b;
-        b.flat = src;
-        b.ld = k;
-        if (!rc)
-            rc = staged_upload(*lease.r, A->device, b, d_dst, 0, (int)n_rows, k, (cudaStream_t)stream);
-        if (rc)
-            return rc;
-        SPMM_CUDA(cudaStreamSynchronize((cudaStream_t)stream)); // before the ring goes back to the free list
-        return SPMM_OK;
-    }
+    const int rc = upload_block(A, src, n_rows, k, d_dst, (cudaStream_t)stream);
+    if (rc)
+        return rc;
     SPMM_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     return SPMM_OK;
+}
+
+int spmm_csr_update_values_host(spmm_csr_t A, const double *vals)
+{
+    SPMM_REQUIRE(A != nullptr, "handle is NULL");
+    SPMM_REQUIRE(A->owns, "a borrowed handle reads the caller's device array: edit it and call spmm_csr_update_values_device");
+    if (A->nnz == 0)
+        return SPMM_OK;
+    SPMM_REQUIRE(vals != nullptr, "vals is NULL");
+    SPMM_CUDA(cudaSetDevice(A->device));
+    std::lock_guard<std::mutex> guard(A->host_mu);
+    int rc = ensure_streams(A);
+    // Straight into the handle's value array; a pageable source is staged as rows of 4 KB (the ring packs row by row) and
+    // the last nnz % 512 values as one short row. Then the tile layout is refreshed from that array.
+    constexpr int W = 512;
+    const long long full = A->nnz / W, rest = A->nnz % W;
+    if (!rc && full)
+        rc = upload_block(A, vals, full, W, A->d_vals, A->stream);
+    if (!rc && rest)
+        rc = upload_block(A, vals + full * W, 1, (int)rest, A->d_vals + full * W, A->stream);
+    if (!rc)
+        rc = update_values(A, A->d_vals, A->stream);
+    const cudaError_t e = cudaStreamSynchronize(A->stream);
+    if (!rc)
+        SPMM_CUDA(e);
+    return rc;
 }
 
 int spmm_download_dense(spmm_csr_t A, const double *d_src, long long n_rows, int k, double *dst, void *stream)

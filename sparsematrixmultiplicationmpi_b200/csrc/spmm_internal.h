@@ -124,6 +124,7 @@ struct spmm_csr_s
     int *d_tsingles = nullptr;
     int *d_torder = nullptr;          // walking order of the tiles (nullptr: as they lie)
     int tl_stride = 0, tl_group = 0;  // detected far-band distance in rows, planes interleaved per super-group
+    mutable bool tl_refreshed = false; // blob values rewritten since the last tiled launch (that launch is not programmatic)
     // precomputed CTA cuts per (kind, grid size): kind 0 = rows of the CSR
     mutable std::map<long long, int *> bounds;
     // merge-path scratch (carry rows), grown on demand
@@ -147,6 +148,9 @@ bool tiled_shape_ok(const spmm_csr_s *A, const double *d_B, long long ldb, const
 int launch_tiled(const spmm_csr_s *A, const double *d_B, long long ldb, double *d_C, long long ldc, int kc,
                  cudaStream_t stream, const struct ExtraDst *extra = nullptr);
 void free_tiles(spmm_csr_s *A);
+// new values (d_src[nnz], CSR order, on A's device) into A->d_vals (skipped when d_src is A->d_vals) and into the value
+// streams of the tile layout, enqueued on `stream`; the schedule, the CTA cuts and the rest of the layout are kept
+int update_values(spmm_csr_s *A, const double *d_src, cudaStream_t stream);
 int build_tiles(spmm_csr_s *A, int rows_per_tile, int box_rows, int kt_want, int ksplit_want);
 // what AUTO cuts the tile layout for: 64-byte window rows for k <= 8; chunks shared by 2 / 4 CTAs (one k-tile group each) from k = 32 / 64
 inline int tiles_kt_for(int k) { return k <= 8 ? 8 : 16; }

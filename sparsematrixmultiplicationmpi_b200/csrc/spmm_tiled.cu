@@ -554,6 +554,69 @@ __global__ void __launch_bounds__(TB_THREADS) tile_build_kernel(const int *__res
     }
 }
 
+// Value refresh (spmm_csr_update_values_*): new values into the value streams of the blobs, nothing else of the layout
+// changes. One CTA per tile: its unit table says where each row's run starts in the value stream (a split row: its eight
+// segments lie one after the other from the first one's begin), so the table becomes a row -> offset map in shared memory
+// and the tile's non-zeros are then copied in CSR order, coalesced on the source side. Padding slots are left as they are.
+// csr_out != nullptr: the same values also go to the CSR value array (one read of the source, two writes).
+constexpr int TR_THREADS = 256;
+constexpr int TR_U = 4; // loads in flight per thread
+__global__ void __launch_bounds__(TR_THREADS) tile_refresh_kernel(const int *__restrict__ rowptr, const double *__restrict__ src,
+                                                                   double *__restrict__ csr_out, unsigned char *__restrict__ blob,
+                                                                   int n_rows, int T, int hdr_bytes)
+{
+    __shared__ int s_rp[TB_MAXT + 1];
+    __shared__ int s_voff[TB_MAXT];
+    const int t = blockIdx.x;
+    const int r0 = t * T, r1 = min(n_rows, r0 + T), nr = r1 - r0;
+    const int e0 = rowptr[r0];
+    for (int i = threadIdx.x; i <= nr; i += TR_THREADS)
+        s_rp[i] = rowptr[r0 + i] - e0;
+    unsigned char *mine = blob + blob_offset(t, e0, hdr_bytes, T);
+    const int n_units = reinterpret_cast<const int4 *>(mine)->y;
+    const uint2 *units = reinterpret_cast<const uint2 *>(mine + 16);
+    for (int i = threadIdx.x; i < n_units * UW; i += TR_THREADS)
+    {
+        const unsigned w = units[i].x;
+        const int r = (int)((w >> 23) & 0xFF);
+        if (r != (int)UE_PAD_ROW && ((w >> 31) == 0 || i % UW == 0))
+            s_voff[r] = (int)(w & 0x1FFF);
+    }
+    __syncthreads();
+    const int n = s_rp[nr];
+    double *val_out = reinterpret_cast<double *>(mine + hdr_bytes);
+    for (int base = 0; base < n; base += TR_THREADS * TR_U)
+    {
+        double v[TR_U];
+#pragma unroll
+        for (int u = 0; u < TR_U; ++u)
+        {
+            const int j = base + u * TR_THREADS + threadIdx.x;
+            v[u] = j < n ? src[e0 + j] : 0.0;
+        }
+#pragma unroll
+        for (int u = 0; u < TR_U; ++u)
+        {
+            const int j = base + u * TR_THREADS + threadIdx.x;
+            if (j >= n)
+                continue;
+            if (csr_out)
+                csr_out[e0 + j] = v[u];
+            // row holding non-zero j: last local row with s_rp[r] <= j (skips empty rows), as in the builder
+            int lo = 0, hi = nr;
+            while (hi - lo > 1)
+            {
+                const int mid = (lo + hi) >> 1;
+                if (s_rp[mid] <= j)
+                    lo = mid;
+                else
+                    hi = mid;
+            }
+            val_out[s_voff[lo] + (j - s_rp[lo])] = v[u];
+        }
+    }
+}
+
 // ---- PTX helpers: mbarrier, bulk copies -------------------------------------------------------
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count)
@@ -1184,7 +1247,11 @@ int launch_tiled_t(const spmm_csr_s *A, const double *d_B, long long ldb, double
         SPMM_CUDA(cudaMalloc(&d_prof, sizeof(long long) * 12 * 1024));
     a.prof = d_prof;
 #endif
-    if (tuning().tiled_pdl != 0)
+    // The prologue copies the first blob of each CTA before griddepcontrol.wait: after a value refresh this launch must not
+    // start under the tail of the kernels before it.
+    const bool pdl = tuning().tiled_pdl != 0 && !A->tl_refreshed;
+    A->tl_refreshed = false;
+    if (pdl)
     {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)grid);
@@ -1438,6 +1505,22 @@ int launch_tiled(const spmm_csr_s *A, const double *d_B, long long ldb, double *
         return launch_tiled_ncw<32>(A, ncw, u, npw, d_B, ldb, d_C, ldc, kc, stream, x);
     set_error("tiled kernel: k-tile must be 8, 16 or 32");
     return SPMM_ERR_INVALID;
+}
+
+int update_values(spmm_csr_s *A, const double *d_src, cudaStream_t stream)
+{
+    double *csr_out = d_src == A->d_vals ? nullptr : A->d_vals; // the caller edited A's own array: only the layout is behind
+    if (A->tl_T == 0)
+    {
+        if (csr_out)
+            SPMM_CUDA(cudaMemcpyAsync(csr_out, d_src, sizeof(double) * (size_t)A->nnz, cudaMemcpyDeviceToDevice, stream));
+        return SPMM_OK;
+    }
+    tile_refresh_kernel<<<A->tl_tiles, TR_THREADS, 0, stream>>>(A->d_rowptr, d_src, csr_out, A->d_tblob, A->n_rows, A->tl_T,
+                                                                (int)hdr_bytes_of(A->tl_T));
+    SPMM_CUDA(cudaGetLastError());
+    A->tl_refreshed = true;
+    return SPMM_OK;
 }
 
 } // namespace spmm

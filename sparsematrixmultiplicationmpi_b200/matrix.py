@@ -156,6 +156,30 @@ class DeviceCSR:
         _cabi.check(_cabi.lib().spmm_nnz_range_rows(self.handle, nnz_begin, nnz_end, C.byref(a), C.byref(b)))
         return a.value, b.value
 
+    def update_values(self, values, stream: int | None = None) -> None:
+        """New values for the same pattern (nnz float64 in CSR order); the schedule and the tile layout are kept, the
+        values inside the layout are refreshed. Whether the pattern is the same is not checked.
+
+        A C-contiguous numpy array goes up through the handle's pinned staging (spmm_csr_update_values_host) and the
+        call returns when it is done. A contiguous CUDA tensor on the handle's device is enqueued on `stream` (default:
+        the current torch stream) and not waited for (spmm_csr_update_values_device); it may be the handle's own value
+        array edited in place. No reference to `values` is kept."""
+        if isinstance(values, np.ndarray):
+            if values.dtype != np.float64 or values.ndim != 1 or values.size != self.nnz or not values.flags.c_contiguous:
+                raise ValueError(f"values must be a C-contiguous float64 array of {self.nnz} elements")
+            _cabi.check(_cabi.lib().spmm_csr_update_values_host(self.handle, C.c_void_p(values.ctypes.data)))
+            return
+        import torch
+        if not isinstance(values, torch.Tensor):
+            raise ValueError("values must be a numpy array or a CUDA tensor")
+        if (not values.is_cuda or values.device.index != self.device or values.dtype != torch.float64 or values.dim() != 1
+                or values.numel() != self.nnz or not values.is_contiguous()):
+            raise ValueError(f"values must be a contiguous float64 tensor of {self.nnz} elements on cuda:{self.device}")
+        if stream is None:
+            stream = torch.cuda.current_stream(values.device).cuda_stream
+        _cabi.check(_cabi.lib().spmm_csr_update_values_device(self.handle, C.c_void_p(values.data_ptr()),
+                                                              C.c_void_p(stream)))
+
     # -- multiply: device pointers (ints), everything on self.device --
     def multiply(self, d_B: int, k: int, d_C: int, kernel: str = "auto", stream: int = 0) -> None:
         _cabi.check(_cabi.lib().spmm_multiply_device(self.handle, d_B, k, d_C, _cabi.KERNELS[kernel], stream))

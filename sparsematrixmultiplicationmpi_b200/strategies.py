@@ -74,6 +74,10 @@ class CudaCompute:
     def upload(self, m: SparseMatrix) -> DeviceCSR:
         return DeviceCSR.from_host(m, self.index)
 
+    def update_values(self, A: DeviceCSR, values: np.ndarray) -> None:
+        """New values (host, CSR order) for a shard made by upload(): its schedule and tile layout are kept."""
+        A.update_values(values)
+
     def multiply(self, A: DeviceCSR, B: torch.Tensor, k: int, out: torch.Tensor | None = None) -> torch.Tensor:
         """out[n_rows, k] = A * B[n_cols, k]; contiguous float64 tensors on self.device."""
         assert B.is_cuda and B.dtype == torch.float64 and B.is_contiguous()
@@ -112,6 +116,21 @@ class CudaCompute:
         return out
 
 
+def _built_from(plan, m: SparseMatrix):
+    """Record the size of the matrix a plan was made from (from_host), for update_values."""
+    plan._source = (m.numRows, m.numCols, m.nnz)
+    return plan
+
+
+def _check_same_size(plan, m: SparseMatrix) -> None:
+    src = getattr(plan, "_source", None)
+    if src is None:
+        raise ValueError("update_values needs a plan made by from_host")
+    if (m.numRows, m.numCols, m.nnz) != src:
+        raise ValueError(f"update_values: matrix is {m.numRows} x {m.numCols} with {m.nnz} non-zeros, "
+                         f"the plan was made from {src[0]} x {src[1]} with {src[2]}")
+
+
 def _gather_rows_to_root(local: torch.Tensor, counts: list[int], k: int, group=None) -> torch.Tensor | None:
     """Gatherv of row blocks to rank 0 (RowWise.cpp:85-87): equal-size padded blocks, trimmed at the root."""
     rank, P = world(group)
@@ -145,7 +164,14 @@ class RowWise:
     def from_host(cls, compute, m: SparseMatrix, k: int, group=None) -> "RowWise":
         rank, P = world(group)
         s, e = partition_rows(m.numRows, P, rank)
-        return cls(compute, m.numRows, k, compute.upload(m.row_block(s, e)), group)
+        return _built_from(cls(compute, m.numRows, k, compute.upload(m.row_block(s, e)), group), m)
+
+    def update_values(self, m: SparseMatrix) -> None:
+        """New values of the matrix from_host was given: same pattern (the caller's promise, not checked), same size
+        (checked). Every rank refreshes its block in place, schedule and tile layout kept; no collective, since every rank
+        holds the whole host matrix (as main.cpp leaves it)."""
+        _check_same_size(self, m)
+        self.compute.update_values(self.A, m.values[m.rowPtr[self.start]:m.rowPtr[self.end]])
 
     def broadcast_B(self, B: torch.Tensor) -> torch.Tensor:
         """B replicated from rank 0 (main.cpp:137 does this with MPI_Bcast, outside the timed region)."""
@@ -348,7 +374,14 @@ class ColumnBlocks:
         keep = (m.colIndices >= c0) & (m.colIndices < c1)
         csum = np.concatenate(([0], np.cumsum(keep, dtype=np.int64)))
         local = SparseMatrix(m.values[keep], m.colIndices[keep] - c0, csum[m.rowPtr].astype(np.int32), m.numRows, c1 - c0)
-        return cls(compute, m.numRows, m.numCols, k, compute.upload(local), group)
+        return _built_from(cls(compute, m.numRows, m.numCols, k, compute.upload(local), group), m)
+
+    def update_values(self, m: SparseMatrix) -> None:
+        """New values of the matrix from_host was given (same pattern, not checked; same size, checked): this rank's column
+        block takes the values of its columns, cut from the host matrix as from_host cut them."""
+        _check_same_size(self, m)
+        keep = (m.colIndices >= self.col_start) & (m.colIndices < self.col_end)
+        self.compute.update_values(self.A, m.values[keep])
 
     def local_B(self, B_full: torch.Tensor) -> torch.Tensor:
         return B_full[self.col_start:self.col_end].contiguous()
@@ -498,7 +531,13 @@ class ColumnSlabs:
 
     @classmethod
     def from_host(cls, compute, m: SparseMatrix, k: int, group=None) -> "ColumnSlabs":
-        return cls(compute, k, compute.upload(m), group)
+        return _built_from(cls(compute, k, compute.upload(m), group), m)
+
+    def update_values(self, m: SparseMatrix) -> None:
+        """New values of the matrix from_host was given (same pattern, not checked; same size, checked): every rank holds
+        the whole matrix and takes all of them."""
+        _check_same_size(self, m)
+        self.compute.update_values(self.A, m.values)
 
     def run(self, B: torch.Tensor) -> torch.Tensor | None:
         n = self.A.n_rows
@@ -560,7 +599,14 @@ class NonZeroRanges:
     def from_host(cls, compute, m: SparseMatrix, k: int, group=None) -> "NonZeroRanges":
         rank, P = world(group)
         local, first, last, mid = cls.shard_of(m, P, rank)
-        return cls(compute, m.numRows, k, compute.upload(local), first, last, mid, group)
+        return _built_from(cls(compute, m.numRows, k, compute.upload(local), first, last, mid, group), m)
+
+    def update_values(self, m: SparseMatrix) -> None:
+        """New values of the matrix from_host was given (same pattern, not checked; same size, checked): this rank's range
+        of the non-zero stream, the elements from_host gave it."""
+        _check_same_size(self, m)
+        b, e = partition_nnz(m.nnz, self.P, self.rank)
+        self.compute.update_values(self.A, m.values[b:e])
 
     def multiply_local(self, B: torch.Tensor) -> torch.Tensor:
         return self.compute.multiply(self.A, B, self.k)
