@@ -12,6 +12,10 @@
  * layout of the reference's serialize() (utils.cpp:216-228). "d_" arguments
  * are device pointers on the handle's device; all others are host pointers.
  * `stream` is a cudaStream_t passed as void* (NULL = legacy default stream).
+ * Device multiplies of one handle may be enqueued on different streams: the scratch a launch writes on the handle (the
+ * merge kernel's carry rows) is ordered across streams by the library; the operands B and C are the caller's to order.
+ * One handle must not be used from several host threads at once (AUTO's lazy tile layout and the CTA-cut cache are
+ * updated without a lock); the host-buffer forms alone serialize themselves.
  */
 #ifndef SPMM_B200_H
 #define SPMM_B200_H

@@ -370,6 +370,8 @@ int spmm_csr_destroy(spmm_csr_t A)
     cudaFree(A->d_C);
     cudaFree(A->d_carry);
     cudaFree(A->d_carry_row);
+    if (A->carry_done)
+        cudaEventDestroy(A->carry_done);
     if (A->stream)
         cudaStreamDestroy(A->stream);
     if (A->stream_up)

@@ -187,6 +187,9 @@ int launch_merge(spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, lo
     const long long n_teams = std::max(1LL, (total + items - 1) / items);
     const int ldcarry = s.tiles * s.kl * s.nv * s.w;
 
+    // the carry slots are the handle's: a merge multiply on another stream than the last one waits for that one's fix-up
+    if (A->carry_done && A->carry_stream != stream)
+        SPMM_CUDA(cudaStreamWaitEvent(stream, A->carry_done, 0));
     const size_t need_elems = (size_t)(2 * n_teams) * (size_t)ldcarry;
     if (A->carry_elems < need_elems)
     {
@@ -227,8 +230,15 @@ int launch_merge(spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, lo
     args.carry_row = A->d_carry_row;
     args.ldcarry = ldcarry;
     note_kernel("spmm_merge_kernel");
-    return s.w == 2 ? launch_merge_w2(s.kl, s.nv, u, args, s.tiles, stream)
-                    : launch_merge_w1(s.kl, s.nv, u, args, s.tiles, stream);
+    const int rc = s.w == 2 ? launch_merge_w2(s.kl, s.nv, u, args, s.tiles, stream)
+                            : launch_merge_w1(s.kl, s.nv, u, args, s.tiles, stream);
+    if (rc != SPMM_OK)
+        return rc;
+    if (!A->carry_done)
+        SPMM_CUDA(cudaEventCreateWithFlags(&A->carry_done, cudaEventDisableTiming));
+    SPMM_CUDA(cudaEventRecord(A->carry_done, stream));
+    A->carry_stream = stream;
+    return SPMM_OK;
 }
 
 } // namespace spmm

@@ -127,10 +127,13 @@ struct spmm_csr_s
     mutable bool tl_refreshed = false; // blob values rewritten since the last tiled launch (that launch is not programmatic)
     // precomputed CTA cuts per (kind, grid size): kind 0 = rows of the CSR
     mutable std::map<long long, int *> bounds;
-    // merge-path scratch (carry rows), grown on demand
+    // merge-path scratch (carry rows), grown on demand; one set per handle, so merge multiplies enqueued on different streams
+    // are ordered through carry_done (recorded after each fix-up) whenever the stream changes
     double *d_carry = nullptr;
     int *d_carry_row = nullptr;
     size_t carry_elems = 0, carry_rows = 0;
+    cudaEvent_t carry_done = nullptr;
+    cudaStream_t carry_stream = nullptr; // stream of the last merge launch (carry_done was recorded there)
 };
 
 namespace spmm
