@@ -282,7 +282,10 @@ int spmm_gen_fat_vector_device(int device, double *d_out, long long n_elems, lon
                                unsigned long long seed, void *stream);
 
 /* Measurement knob (not needed for correct results): override the automatic team shape.
- * keys: rows.kl rows.nv rows.np rows.unroll rows.vec rows.ctas_per_sm merge.items tiled tiled.kt tiled.ncw tiled.unroll tiled.thr tiled.chunk tiled.depth tiled.pool tiled.ns tiled.ksplit tiled.npw tiled.prefetch host.slabs reset */
+ * keys: rows.kl rows.nv rows.np rows.unroll rows.vec rows.ctas_per_sm rows.tile rows.prefetch merge.items merge.wave
+ *       tiled tiled.thr tiled.chunk tiled.depth tiled.pool tiled.ns tiled.ksplit tiled.group tiled.stride tiled.pdl
+ *       tiled.auto_after stream stream.tile stream.kmax stream.min_nnz host.slabs reset
+ * An unknown key fails with SPMM_ERR_INVALID. */
 int spmm_tune_set(const char *key, int value);
 
 #ifdef __cplusplus

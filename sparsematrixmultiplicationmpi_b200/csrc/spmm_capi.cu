@@ -241,22 +241,16 @@ int spmm_tune_set(const char *key, int value)
     if (k == "rows.np") t.rows_np = value;
     else if (k == "rows.kl") t.rows_kl = value;
     else if (k == "rows.nv") t.rows_nv = value;
-    else if (k == "rows.sweep") t.rows_sweep = value;
     else if (k == "rows.prefetch") t.rows_prefetch = value;
     else if (k == "rows.tile") t.rows_tile = value;
     else if (k == "tiled") t.tiled = value;
-    else if (k == "tiled.kt") t.tiled_kt = value;
-    else if (k == "tiled.ncw") t.tiled_ncw = value;
-    else if (k == "tiled.unroll") t.tiled_unroll = value;
     else if (k == "tiled.thr") t.tiled_thr = value;
     else if (k == "tiled.chunk") t.tiled_chunk = value;
     else if (k == "tiled.depth") t.tiled_depth = value;
     else if (k == "tiled.pool") t.tiled_pool = value;
     else if (k == "tiled.ns") t.tiled_ns = value;
     else if (k == "tiled.ksplit") t.tiled_ksplit = value;
-    else if (k == "tiled.npw") t.tiled_npw = value;
     else if (k == "host.slabs") t.host_slabs = value;
-    else if (k == "tiled.prefetch") t.tiled_prefetch = value;
     else if (k == "tiled.group") t.tiled_group = value;
     else if (k == "tiled.pdl") t.tiled_pdl = value;
     else if (k == "tiled.auto_after") t.tiled_auto_after = value;
@@ -265,7 +259,6 @@ int spmm_tune_set(const char *key, int value)
     else if (k == "stream.tile") t.stream_tile = value;
     else if (k == "stream.kmax") t.stream_auto_kmax = value;
     else if (k == "stream.min_nnz") t.stream_auto_min_nnz = value;
-    else if (k == "rows.threads") t.rows_threads = value;
     else if (k == "rows.unroll") t.rows_unroll = value;
     else if (k == "rows.vec") t.rows_vec = value;
     else if (k == "rows.ctas_per_sm") t.rows_ctas_per_sm = value;
@@ -461,8 +454,7 @@ static void auto_tile_layout(spmm_csr_t A, int k)
     if (A->auto_calls++ < tuning().tiled_auto_after)
         return;
     A->tl_tried = true;
-    const int brc = build_tiles(A, -1, 0, tuning().tiled_kt > 0 ? tuning().tiled_kt : tiles_kt_for(k),
-                                tuning().tiled_ksplit > 0 ? tuning().tiled_ksplit : tiles_ksplit_for(k));
+    const int brc = build_tiles(A, -1, 0, tiles_kt_for(k), tuning().tiled_ksplit > 0 ? tuning().tiled_ksplit : tiles_ksplit_for(k));
     A->tl_auto = true;
     if (brc != SPMM_OK)
         free_tiles(A);

@@ -122,9 +122,6 @@ int launch_rows(const spmm_csr_s *A, int row_begin, int row_end, long long nnz_l
     // in L2 / L1 (cfg2): 2 is the measured optimum for wide pieces
     const bool b_beyond_l2 = (long long)A->n_cols * kc * 8 > device_props(A->device).l2_bytes;
     int u = t.rows_unroll > 0 ? t.rows_unroll : (np >= 8 ? 1 : np >= 2 ? 2 : (s.nv >= 4 ? (b_beyond_l2 ? 4 : 2) : 4));
-    const bool sweep = t.rows_sweep > 0 && s.w == 2;
-    if (sweep && t.rows_np > 0)
-        np = std::max(1, std::min(t.rows_np, 32 / s.kl)); // sweep shapes allow NP > 1 with NV > 1
 
     SpmmArgs args = {};
     if (extra)
@@ -142,20 +139,11 @@ int launch_rows(const spmm_csr_s *A, int row_begin, int row_end, long long nnz_l
     args.nnz_hi = (int)nnz_hi;
     args.c_row0 = c_row0;
     args.kc = kc;
-    args.tiles = s.tiles;
     // L2 prefetch only when the operands are 16-byte aligned, B is one contiguous block that starts
     // at column 0 of its rows (no k-slab), and the A arrays are the handle's own (padded) allocations
     const bool aligned = ((uintptr_t)A->d_colidx % 16 == 0) && ((uintptr_t)A->d_vals % 16 == 0) && ((uintptr_t)d_B % 16 == 0);
     args.prefetch = aligned ? (t.rows_prefetch >= 0 ? t.rows_prefetch : 3) : 0;
     args.b_bytes = (ldb == kc && !t_b_is_window) ? (long long)A->n_cols * ldb * 8 : 0;
-    if (sweep)
-    {
-        note_kernel("spmm_rows_sweep_kernel");
-        const int rc = launch_sweep_w2(A, s.kl, s.nv, np, u, t.rows_threads > 0 ? t.rows_threads : 512, args, s.tiles,
-                                       A->device, stream);
-        if (rc != -1)
-            return rc;
-    }
     note_kernel("spmm_rows_kernel");
     return s.w == 2 ? launch_rows_w2(A, s.kl, s.nv, np, u, args, s.tiles, A->device, stream)
                     : launch_rows_w1(A, s.kl, s.nv, np, u, args, s.tiles, A->device, stream);

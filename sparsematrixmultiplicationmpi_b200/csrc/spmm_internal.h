@@ -55,21 +55,15 @@ struct Tuning
     int rows_ctas_per_sm = 0;
     int merge_items = 0;    // merge-path items per team
     int merge_wave = 0;     // merge-path: warps per SM the item count is shrunk for on small shards (0 = 64)
-    int rows_sweep = 0;     // 1: one CTA per SM walks the column tiles itself (L1-resident window)
-    int rows_threads = 0;   // sweep kernels: 512 or 1024 threads
     int rows_tile = 0;      // 0 auto, > 0 rows per round-robin tile, -1 never tile (one chunk per CTA)
     int rows_prefetch = -1; // -1 auto; bit0 A chunk, bit1 B share: TMA prefetch into L2 at kernel start
     int tiled = -1;         // -1 auto, 0 never use the tile layout, 1 always when built
-    int tiled_kt = 0;       // tiled kernel: k-tile width (16, 32)
-    int tiled_ncw = 0;      // consumer warps (8, 12, 16)
-    int tiled_unroll = 0;   // records in flight per team (2, 4)
     int tiled_thr = 0;      // build: non-zeros a box needs in a tile to be loaded as a box (else single rows)
     int tiled_chunk = 0;    // build: tiles per chunk
     int tiled_depth = 0;    // build: work items in flight (2..8)
     int tiled_pool = 0;     // build: rows of the singles pool
     int tiled_ns = 0;       // build: cap on the window slots
     int tiled_ksplit = 0;   // build: CTAs that share one chunk, each taking a group of k-tiles (0/1 none)
-    int tiled_npw = 0;      // launch: producer warps (4, 8)
     int host_slabs = 0;     // host-buffer multiply: k-slabs in the PCIe pipeline (0 auto, 1 none)
     int tiled_auto_after = 8; // AUTO builds the tile layout on the multiply after this many whole-matrix multiplies of a handle
                               // (the build costs 4-7 ms of wall clock on cfg2 at k = 16 and 14-25 ms at k = 64 — five device passes of 1.9 ms
@@ -77,7 +71,6 @@ struct Tuning
     int tiled_pdl = 1;      // launch: programmatic dependent launch of the tiled kernel (0 off)
     int tiled_group = 0;    // build: tiles one far-band apart walked in turn, this many bands per group (0 auto = 2, 1 off)
     int tiled_stride = 0;   // build: far-band distance in rows (0 = detect from the matrix)
-    int tiled_prefetch = -1; // launch: tiles ahead whose blob is prefetched into L2 (-1 auto)
     int stream = -1;        // -1 auto, 0 AUTO never uses the stream kernel (k = 1, 2, 4, 8)
     int stream_auto_kmax = 1; // AUTO takes the stream kernel up to this k ...
     int stream_auto_min_nnz = 4 << 20; // ... from this many non-zeros (measured: equal to the row kernel at 2.6 M non-zeros, 43 against 56 us at 10.5 M; profiles/r1_stream.md)

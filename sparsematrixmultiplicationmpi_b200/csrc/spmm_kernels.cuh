@@ -335,7 +335,6 @@ struct SpmmArgs
     int c_row0;             // row id stored at C[0]
     int kc;                 // columns computed
     const int *bounds;      // optional precomputed CTA row cuts (gridDim.x+1 entries)
-    int tiles;              // column tiles (SWEEP kernels walk them in-kernel)
     int tile_rows;          // > 0: CTAs take row tiles of this size round-robin (b, b+grid, ...) instead of one chunk
     int prefetch;           // bit0: CTA prefetches its own A chunk into L2; bit1: its share of B
     long long b_bytes;      // bytes of the B operand (0: not contiguous, no prefetch)
@@ -362,13 +361,8 @@ constexpr int min_blocks(int nv, int w, int u, int rows, int threads)
 // 32/(KL*NP) teams share a warp. Software pipeline: while the U B-row slices of a
 // group are in flight, the column ids / values of the next group and the extent of
 // the team's next row are already being fetched, so a group costs one memory latency.
-//
-// SWEEP=true: one launch row (gridDim.y == 1) walks ALL column tiles of its chunk itself, one
-// after the other, instead of spreading the tiles over blockIdx.y. With one such CTA per SM the
-// SM follows a single stream of consecutive rows on a narrow column tile, which is what keeps
-// the B rows shared by neighbouring rows resident in L1 (DESIGN.md §4.1).
-template <int KL, int NV, int W, int NP, int U, bool FULL, int THREADS, bool SWEEP = false>
-__global__ void __launch_bounds__(THREADS, SWEEP ? 1 : min_blocks(NV, W, U, 1, THREADS)) spmm_rows_kernel(const SpmmArgs a)
+template <int KL, int NV, int W, int NP, int U, bool FULL, int THREADS>
+__global__ void __launch_bounds__(THREADS, min_blocks(NV, W, U, 1, THREADS)) spmm_rows_kernel(const SpmmArgs a)
 {
     constexpr int T = KL * NP;
     constexpr int RW = 32 / T;
@@ -420,9 +414,7 @@ __global__ void __launch_bounds__(THREADS, SWEEP ? 1 : min_blocks(NV, W, U, 1, T
     const int g = lt / KL;   // which of the NP concurrent non-zeros
     const int kl = lt % KL;  // which column group
     const int slot = (threadIdx.x >> 5) * RW + lane / T;
-  for (int tile = SWEEP ? 0 : (int)blockIdx.y; tile < (SWEEP ? a.tiles : (int)blockIdx.y + 1); ++tile)
-  {
-    const int tile0 = tile * S::TILE;
+    const int tile0 = (int)blockIdx.y * S::TILE;
     const unsigned mask = slice_mask<KL, NV, W>(tile0, kl, a.kc);
     const double *__restrict__ Bk = a.B + tile0 + kl * W;
 
@@ -529,7 +521,6 @@ __global__ void __launch_bounds__(THREADS, SWEEP ? 1 : min_blocks(NV, W, U, 1, T
         js = njs;
         je = nje;
     }
-  }
   }
 }
 

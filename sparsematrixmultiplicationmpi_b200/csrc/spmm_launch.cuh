@@ -32,7 +32,7 @@ struct KernelInfo
 // One-time per-kernel set-up: give the whole unified array to L1D (B-row reuse lives
 // there; the kernels use a few bytes of static smem only) and query occupancy.
 template <typename K>
-int kernel_info(K kern, int *ctas_per_sm, int threads = THREADS)
+int kernel_info(K kern, int *ctas_per_sm)
 {
     static std::mutex mu;
     static std::map<std::pair<const void *, int>, KernelInfo> cache; // function attributes and occupancy are per device
@@ -46,7 +46,7 @@ int kernel_info(K kern, int *ctas_per_sm, int threads = THREADS)
     {
         SPMM_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
         KernelInfo ki;
-        SPMM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ki.ctas_per_sm, kern, threads, 0));
+        SPMM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ki.ctas_per_sm, kern, THREADS, 0));
         if (ki.ctas_per_sm < 1)
             ki.ctas_per_sm = 1;
         it = cache.emplace(key, ki).first;
@@ -205,68 +205,6 @@ int launch_rows_shape(const spmm_csr_s *A, int kl, int nv, int np, int u, const 
     set_error("rows kernel: unsupported team shape kl=" + std::to_string(kl) + " nv=" + std::to_string(nv));
     return SPMM_ERR_UNSUPPORTED;
 }
-
-
-// ---- sweep variant: one CTA per SM, column tiles walked in-kernel --------------------------
-template <int KL, int NV, int W, int NP, int U, int TH>
-int launch_sweep_one(const spmm_csr_s *A, const SpmmArgs &args, int tiles, int device, cudaStream_t stream)
-{
-    int rc;
-    SpmmArgs a2 = args;
-    a2.tiles = tiles;
-    a2.bounds = nullptr;
-    a2.tile_rows = 0;
-    const Tuning &t = tuning();
-    const int per_sm = t.rows_ctas_per_sm > 0 ? t.rows_ctas_per_sm : 1;
-    constexpr int SLOTS = (TH / 32) * (32 / (KL * NP));
-    const long long rows = (long long)args.row_end - args.row_begin;
-    long long grid = (long long)device_props(device).sm_count * per_sm;
-    grid = std::max(1LL, std::min(grid, (rows + SLOTS - 1) / SLOTS));
-    auto go = [&](auto kern) -> int {
-        int dummy = 0;
-        int r = kernel_info(kern, &dummy, TH);
-        if (r)
-            return r;
-        if (args.row_begin == 0 && args.row_end == A->n_rows && args.nnz_lo == 0 && args.nnz_hi == A->nnz)
-        {
-            r = cached_bounds(A, 0, (int)grid, stream, &a2.bounds, [&](int *out) {
-                chunk_bounds_kernel<<<((unsigned)grid + 256) / 256, 256, 0, stream>>>(args.rowptr, A->n_rows,
-                                                                                 (int)A->nnz, (int)grid, out);
-            });
-            if (r)
-                return r;
-        }
-        kern<<<dim3((unsigned)grid, 1), TH, 0, stream>>>(a2);
-        SPMM_CUDA(cudaGetLastError());
-        return SPMM_OK;
-    };
-    if (args.kc == tiles * KL * NV * W)
-        rc = go(spmm_rows_kernel<KL, NV, W, NP, U, true, TH, true>);
-    else
-        rc = go(spmm_rows_kernel<KL, NV, W, NP, U, false, TH, true>);
-    return rc;
-}
-
-// shapes offered: KL=8 lanes x NV in {1,2,4} accesses, NP in {1,2,4}, U in {2,4}; 512 or 1024 threads
-template <int W>
-int launch_sweep_shape(const spmm_csr_s *A, int kl, int nv, int np, int u, int threads, const SpmmArgs &a, int tiles,
-                       int dev, cudaStream_t s)
-{
-#define SPMM_SW_CASE(N, P, UU)                                                                  \
-    if (kl == 8 && nv == N && np == P && u == UU)                                               \
-    {                                                                                           \
-        if (threads >= 1024)                                                                    \
-            return launch_sweep_one<8, N, W, P, UU, 1024>(A, a, tiles, dev, s);                 \
-        return launch_sweep_one<8, N, W, P, UU, 512>(A, a, tiles, dev, s);                      \
-    }
-    SPMM_SW_CASE(1, 1, 2) SPMM_SW_CASE(1, 1, 4) SPMM_SW_CASE(1, 2, 2) SPMM_SW_CASE(1, 2, 4) SPMM_SW_CASE(1, 4, 2) SPMM_SW_CASE(1, 4, 4)
-    SPMM_SW_CASE(2, 1, 2) SPMM_SW_CASE(2, 1, 4) SPMM_SW_CASE(2, 2, 2) SPMM_SW_CASE(2, 2, 4) SPMM_SW_CASE(2, 4, 2) SPMM_SW_CASE(2, 4, 4)
-    SPMM_SW_CASE(4, 1, 2) SPMM_SW_CASE(4, 1, 4) SPMM_SW_CASE(4, 2, 2) SPMM_SW_CASE(4, 2, 4) SPMM_SW_CASE(4, 4, 2) SPMM_SW_CASE(4, 4, 4)
-#undef SPMM_SW_CASE
-    return -1;
-}
-int launch_sweep_w2(const spmm_csr_s *A, int kl, int nv, int np, int u, int threads, const SpmmArgs &a, int tiles, int dev,
-                    cudaStream_t s);
 
 // ---- merge-path ---------------------------------------------------------------------
 template <int KL, int NV, int W, int U, bool FULL>

@@ -712,7 +712,7 @@ struct TiledArgs
     const double *B;
     double *C;
     long long ldb, ldc;
-    int n_tiles, n_chunks /* shares: chunks x ksplit */, ksplit, tiles_per_chunk, T, BR, NS, POOL, kc, nkt, depth, prefetch;
+    int n_tiles, n_chunks /* shares: chunks x ksplit */, ksplit, tiles_per_chunk, T, BR, NS, POOL, kc, nkt, depth;
     unsigned hdr_bytes;   // header + unit table bytes of a blob
     unsigned blob_stride; // bytes reserved per blob buffer in smem
     unsigned slab_off;    // offset of the slab (window slots, then the singles pool) from the aligned smem base
@@ -853,18 +853,6 @@ __global__ void __launch_bounds__((NCW + NPW) * 32, 1) spmm_tiled_kernel(const T
                 mbar_expect_tx(bar, T_NO_STAGE ? m.d.bytes
                                                : m.d.bytes + (unsigned)n_loads * box_bytes + (unsigned)n_singles * (KT * 8));
                 bulk_g2s(s_blob + st * a.blob_stride, a.blob + ((unsigned long long)m.d.off16 << 4), m.d.bytes, bar);
-            }
-            if (pw == 1 && lane == 0 && a.prefetch > 0)
-            {
-                // the blob of the item `prefetch` tiles further down the chunk: into L2 now, so that its copy later is an L2 hit
-                const int tp = cur.t + a.prefetch;
-                if (tp < cur.t_end)
-                {
-                    const TileDesc dp = a.tdesc[tp];
-                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.blob + ((unsigned long long)dp.off16 << 4)),
-                                 "r"(dp.bytes)
-                                 : "memory");
-                }
             }
             if (w == 0)
                 asm volatile("griddepcontrol.wait;" ::: "memory"); // B may be the result of the kernel before this one
@@ -1194,7 +1182,7 @@ int launch_tiled_t(const spmm_csr_s *A, const double *d_B, long long ldb, double
     const TiledSmem m = tiled_smem(KT, A->tl_depth, A->tl_T, A->tl_BR, A->tl_NS, A->tl_POOL, A->tl_max_blob);
     if (m.total > (size_t)SMEM_CAP)
     {
-        set_error("tiled kernel: the tile layout was built for a narrower k-tile; it does not fit in shared memory");
+        set_error("tiled kernel: the tile layout does not fit in shared memory");
         return SPMM_ERR_UNSUPPORTED;
     }
     static std::mutex mu;
@@ -1235,7 +1223,6 @@ int launch_tiled_t(const spmm_csr_s *A, const double *d_B, long long ldb, double
     a.kc = kc;
     a.nkt = (kc + KT - 1) / KT;
     a.depth = A->tl_depth;
-    a.prefetch = tuning().tiled_prefetch >= 0 ? tuning().tiled_prefetch : 0;
     a.hdr_bytes = hdr_bytes_of(A->tl_T);
     a.blob_stride = (unsigned)m.blob_stride;
     a.slab_off = (unsigned)m.slab_off;
@@ -1285,37 +1272,6 @@ int launch_tiled_t(const spmm_csr_s *A, const double *d_B, long long ldb, double
     }
 #endif
     return SPMM_OK;
-}
-
-template <int KT>
-int launch_tiled_ncw(const spmm_csr_s *A, int ncw, int u, int npw, const double *d_B, long long ldb, double *d_C,
-                     long long ldc, int kc, cudaStream_t s, const ExtraDst &x)
-{
-    if (npw == 8)
-    {
-        if (ncw == 12 && u == 4)
-            return launch_tiled_t<KT, 12, 4, 8>(A, d_B, ldb, d_C, ldc, kc, s, x);
-        if (ncw == 16 && u == 4)
-            return launch_tiled_t<KT, 16, 4, 8>(A, d_B, ldb, d_C, ldc, kc, s, x);
-        set_error("tiled kernel: 8 producer warps go with 12 or 16 consumer warps and unroll 4");
-        return SPMM_ERR_INVALID;
-    }
-#define SPMM_TILED_CASE(N, UU) \
-    if (ncw == N && u == UU)   \
-        return launch_tiled_t<KT, N, UU, 4>(A, d_B, ldb, d_C, ldc, kc, s, x);
-    SPMM_TILED_CASE(4, 4)
-    SPMM_TILED_CASE(4, 8)
-    SPMM_TILED_CASE(8, 4)
-    SPMM_TILED_CASE(8, 8)
-    SPMM_TILED_CASE(12, 4)
-    SPMM_TILED_CASE(12, 8)
-    SPMM_TILED_CASE(16, 4)
-    SPMM_TILED_CASE(16, 8)
-    SPMM_TILED_CASE(20, 4)
-    SPMM_TILED_CASE(24, 4)
-#undef SPMM_TILED_CASE
-    set_error("tiled kernel: consumer warps x unroll must be one of 4x4 4x8 8x4 8x8 12x4 12x8 16x4 16x8 20x4 24x4");
-    return SPMM_ERR_INVALID;
 }
 
 struct BuildResult
@@ -1482,29 +1438,11 @@ int launch_tiled(const spmm_csr_s *A, const double *d_B, long long ldb, double *
                  cudaStream_t stream, const ExtraDst *extra)
 {
     const ExtraDst x = extra ? *extra : ExtraDst();
-    const Tuning &t = tuning();
     note_kernel("spmm_tiled_kernel");
-    const int kt = t.tiled_kt > 0 ? t.tiled_kt : A->tl_kt;
-    const int ncw = t.tiled_ncw > 0 ? t.tiled_ncw : 16;
-    const int u = t.tiled_unroll > 0 ? t.tiled_unroll : 4;
-    const int npw = t.tiled_npw == 8 ? 8 : 4;
-    if (kt == 8)
-    {
-        if (ncw == 16 && u == 4 && npw == 4)
-            return launch_tiled_t<8, 16, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
-        if (ncw == 12 && u == 4 && npw == 4)
-            return launch_tiled_t<8, 12, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
-        if (ncw == 8 && u == 4 && npw == 4)
-            return launch_tiled_t<8, 8, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
-        set_error("tiled kernel: the 8-column k-tile goes with 8, 12 or 16 consumer warps, unroll 4, 4 producer warps");
-        return SPMM_ERR_INVALID;
-    }
-    if (kt == 16)
-        return launch_tiled_ncw<16>(A, ncw, u, npw, d_B, ldb, d_C, ldc, kc, stream, x);
-    if (kt == 32)
-        return launch_tiled_ncw<32>(A, ncw, u, npw, d_B, ldb, d_C, ldc, kc, stream, x);
-    set_error("tiled kernel: k-tile must be 8, 16 or 32");
-    return SPMM_ERR_INVALID;
+    // the kernel's shape is the one the layout was cut for
+    if (A->tl_kt == 8)
+        return launch_tiled_t<8, 16, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
+    return launch_tiled_t<16, 16, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
 }
 
 int update_values(spmm_csr_s *A, const double *d_src, cudaStream_t stream)
@@ -1527,7 +1465,8 @@ int update_values(spmm_csr_s *A, const double *d_src, cudaStream_t stream)
 
 namespace spmm
 {
-// kt_want / ksplit_want: k-tile width and CTAs per chunk the layout is cut for (0 = the tuning knob, else its default).
+// kt_want: k-tile width the layout is cut for, 8 or 16 (0 = 16), the two widths the tiled kernel is built for.
+// ksplit_want: CTAs per chunk (0 = the tuning knob, else its default).
 // Explicit parameters, not the process-wide tuning: concurrent multiplies of rank-threads build their layouts side by side.
 int build_tiles(spmm_csr_t A, int rows_per_tile, int box_rows, int kt_want, int ksplit_want)
 {
@@ -1537,6 +1476,7 @@ int build_tiles(spmm_csr_t A, int rows_per_tile, int box_rows, int kt_want, int 
                  "rows_per_tile must be 0 (drop), -1 (auto) or a multiple of 8 in [8, 248]");
     SPMM_REQUIRE(box_rows == 0 || box_rows == 4 || box_rows == 8 || box_rows == 16 || box_rows == 32,
                  "box_rows must be 0 (auto), 4, 8, 16 or 32");
+    SPMM_REQUIRE(kt_want == 0 || kt_want == 8 || kt_want == 16, "k-tile must be 0 (auto), 8 or 16");
     SPMM_CUDA(cudaSetDevice(A->device));
     free_tiles(A);
     A->tl_tried = true; // an explicit call (build or drop) settles it: AUTO does not try again
@@ -1545,7 +1485,7 @@ int build_tiles(spmm_csr_t A, int rows_per_tile, int box_rows, int kt_want, int 
         return SPMM_OK;
     const Tuning &tn = tuning();
     const int BR = box_rows ? box_rows : 16;
-    const int kt = kt_want > 0 ? kt_want : (tn.tiled_kt > 0 ? tn.tiled_kt : 16); // k-tile the window is sized for
+    const int kt = kt_want ? kt_want : 16; // k-tile the window is sized for
     const int sms = device_props(A->device).sm_count;
     // measured on the cop20k_A shape (profiles/r1_tiled.md): tall tiles and a wide window beat a deeper pipeline
     const int kt_for_depth = kt;

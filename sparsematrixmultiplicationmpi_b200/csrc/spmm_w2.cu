@@ -6,11 +6,6 @@ int launch_rows_w2(const spmm_csr_s *A, int kl, int nv, int np, int u, const Spm
 {
     return launch_rows_shape<2>(A, kl, nv, np, u, a, tiles, dev, s);
 }
-int launch_sweep_w2(const spmm_csr_s *A, int kl, int nv, int np, int u, int threads, const SpmmArgs &a, int tiles, int dev,
-                    cudaStream_t s)
-{
-    return launch_sweep_shape<2>(A, kl, nv, np, u, threads, a, tiles, dev, s);
-}
 int launch_merge_w2(int kl, int nv, int u, const SpmmArgs &a, int tiles, cudaStream_t s)
 {
     return launch_merge_shape<2>(kl, nv, u, a, tiles, s);

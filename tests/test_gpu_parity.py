@@ -418,18 +418,6 @@ def test_strategy_classes_on_one_gpu(oracle):
     assert_close_rel(spmm.NonZeroRanges.from_host(eng, m, 16).run(dB).cpu().numpy(), seq, tol=REL_TOL)
 
 
-@pytest.mark.parametrize("nv,np_,u,th", [(1, 1, 2, 512), (1, 4, 4, 1024), (2, 2, 2, 512), (2, 4, 4, 512), (4, 1, 4, 512),
-                                          (4, 2, 2, 1024), (4, 4, 4, 1024), (2, 1, 4, 1024)])
-@pytest.mark.parametrize("k", [64, 96, 16])
-def test_sweep_kernel_variants(oracle, nv, np_, u, th, k):
-    """One CTA per SM walking the column tiles in-kernel (rows.sweep), incl. ragged last tile (k=96 at nv=4)."""
-    rp, ci, va = random_csr(21, 3000, 3000, 20, long_row=900, empty_every=13, positive=True)
-    B = np.random.default_rng(k).integers(1, 101, (3000, k)).astype(np.float64)
-    tune = {"rows.sweep": 1, "rows.kl": 8, "rows.nv": nv, "rows.np": np_, "rows.unroll": u, "rows.threads": th}
-    got = gpu_multiply(spmm.SparseMatrix(va, ci, rp, 3000, 3000), B, k, "rows", tune)
-    assert_close_rel(got, oracle.spmm(rp, ci, va, B, k), tol=REL_TOL)
-
-
 @pytest.mark.parametrize("tile", [32, 100, 4096])
 @pytest.mark.parametrize("k", [1, 16, 64])
 def test_round_robin_row_tiles(oracle, tile, k):
@@ -495,14 +483,13 @@ def test_tiled_kernel_vs_oracle(oracle, shape, k):
 
 
 @pytest.mark.parametrize("T,BR", [(8, 4), (16, 16), (64, 8), (64, 32), (128, 16), (248, 16)])
-@pytest.mark.parametrize("tune", [{}, {"tiled.kt": 32}, {"tiled.kt": 32, "tiled.ncw": 12, "tiled.depth": 2},
-                                  {"tiled.ncw": 16, "tiled.unroll": 8, "tiled.depth": 8}, {"tiled.ncw": 4, "tiled.unroll": 8},
-                                  {"tiled.thr": 1, "tiled.chunk": 3}, {"tiled.thr": 100, "tiled.depth": 3},
-                                  {"tiled.ksplit": 2}, {"tiled.ksplit": 4, "tiled.kt": 32}, {"tiled.ksplit": 3, "tiled.chunk": 5}])
+@pytest.mark.parametrize("tune", [{}, {"tiled.depth": 2}, {"tiled.depth": 8}, {"tiled.thr": 1, "tiled.chunk": 3},
+                                  {"tiled.thr": 100, "tiled.depth": 3}, {"tiled.ksplit": 2}, {"tiled.ksplit": 4},
+                                  {"tiled.ksplit": 3, "tiled.chunk": 5}])
 def test_tiled_shapes_and_teams(oracle, T, BR, tune):
-    """Explicit tile heights / box heights x k-tile, warps, pipeline depth, box threshold (all boxes .. all single
-    rows), chunk length: split rows (the 900-long row: 8 segments folded by shuffles), empty rows, ragged last
-    tile and k-tile (k=48 with k-tile 32), window wrap-around across passes."""
+    """Explicit tile heights / box heights x pipeline depth, box threshold (all boxes .. all single rows), chunk
+    length, CTAs per chunk: split rows (the 900-long row: 8 segments folded by shuffles), empty rows, ragged last
+    tile, window wrap-around across passes. Ragged k-tiles are covered by test_tiled_kernel_vs_oracle (k = 30, 100)."""
     n, k = 3003, 48
     rp, ci, va = banded_csr(37, n, 14, 16, (-200, 0, 200), 900, 11)
     B = np.random.default_rng(3).integers(1, 101, (n, k)).astype(np.float64)
@@ -517,28 +504,25 @@ def test_tiled_shapes_and_teams(oracle, T, BR, tune):
 
 @pytest.mark.parametrize("shape", list(TILED_SHAPES))
 @pytest.mark.parametrize("k", [2, 6, 8])
-@pytest.mark.parametrize("ncw", [16, 8])
-def test_tiled_kernel_8_column_k_tile(oracle, shape, k, ncw):
-    """k <= 8: the window rows are 64 bytes (k-tile of 8 columns, one 16-byte access per lane)."""
+def test_tiled_kernel_8_column_k_tile(oracle, shape, k):
+    """k <= 8: the window rows are 64 bytes (k-tile of 8 columns, one 16-byte access per lane). The layout is cut for k
+    as AUTO cuts it, and the tiled kernel runs with the k-tile of the layout."""
     n, mean, hb, planes, long_row, ee = TILED_SHAPES[shape]
     rp, ci, va = banded_csr(33, n, mean, hb, planes, long_row, ee)
     B = np.random.default_rng(k).integers(1, 101, (n, k)).astype(np.float64)
     ref = oracle.spmm(rp, ci, va, B, k)
     _cabi.tune("reset", 0)
-    _cabi.tune("tiled.kt", 8)
-    _cabi.tune("tiled.ncw", ncw)
-    try:
-        with spmm.DeviceCSR.from_host(spmm.SparseMatrix(va, ci, rp, n, n), 0) as A:
-            info = A.build_tiles(-1, 0)
-            if not info["rows_per_tile"]:
-                pytest.skip("no tile shape fits this matrix")
-            dB = dev(B)
-            dC = torch.full((n, k), np.nan, dtype=torch.float64, device="cuda")
-            A.multiply(dB.data_ptr(), k, dC.data_ptr(), "tiled", torch.cuda.current_stream().cuda_stream)
-            torch.cuda.synchronize()
-            got = dC.cpu().numpy()
-    finally:
-        _cabi.tune("reset", 0)
+    with spmm.DeviceCSR.from_host(spmm.SparseMatrix(va, ci, rp, n, n), 0) as A:
+        info = A.build_tiles(-1, 0, k)
+        if not info["rows_per_tile"]:
+            pytest.skip("no tile shape fits this matrix")
+        dB = dev(B)
+        dC = torch.full((n, k), np.nan, dtype=torch.float64, device="cuda")
+        A.multiply(dB.data_ptr(), k, dC.data_ptr(), "tiled", torch.cuda.current_stream().cuda_stream)
+        torch.cuda.synchronize()
+        got = dC.cpu().numpy()
+        assert A.tile_info()["rows_per_tile"] > 0
+        assert _cabi.lib().spmm_last_kernel_name() == b"spmm_tiled_kernel"
     assert_close_rel(got, ref, tol=REL_TOL)
 
 

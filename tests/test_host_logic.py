@@ -19,6 +19,14 @@ def test_partitions_equal_oracle(oracle, total, P):
         assert spmm.partition_nnz(total, P, r) == oracle.partition("nnz", total, P, r) == _cabi.partition_nnz(total, P, r)
 
 
+def test_retired_tuning_keys_are_rejected():
+    """Keys of kernel variants that were removed fail loudly instead of being ignored."""
+    for key, value in (("rows.sweep", 1), ("tiled.kt", 32)):
+        with pytest.raises(_cabi.SpmmError) as e:
+            _cabi.tune(key, value)
+        assert e.value.status == _cabi.SPMM_ERR_INVALID
+
+
 def test_generate_fat_vector_is_the_reference_sequence(golden_multiply):
     assert np.array_equal(spmm.generateLargeFatVector(4, 3), golden_multiply["kat_B"])
     assert np.array_equal(spmm.generateLargeFatVector(7, 5), golden_multiply["fatvec_7x5"])

@@ -118,25 +118,9 @@ def variant_list(k, full):
         for np_ in (1, 2, 4, 8, 16, 32):
             for u in (1, 2, 4):
                 v.append((f"rows np={np_} u={u}", "rows", {"rows.np": np_, "rows.unroll": u}))
-    if k >= 16:
-        for nv in (1, 2, 4):
-            if (k // 2) % (8 * nv):
-                continue
-            for np_ in (1, 2, 4):
-                for u in (2, 4):
-                    for th in (512, 1024):
-                        for ctas in ((1, 2) if th == 512 else (1,)):
-                            v.append((f"sweep nv={nv} np={np_} u={u} th={th} ctas={ctas}", "rows",
-                                      {"rows.sweep": 1, "rows.kl": 8, "rows.nv": nv, "rows.np": np_, "rows.unroll": u,
-                                       "rows.threads": th, "rows.ctas_per_sm": ctas}))
     for pf in (0, 1, 2, 3):
         v.append((f"rows pf={pf}", "rows", {"rows.prefetch": pf}))
         v.append((f"rows u=4 pf={pf}", "rows", {"rows.prefetch": pf, "rows.unroll": 4}))
-        if k >= 16 and (k // 2) % 32 == 0:
-            v.append((f"sweep nv=4 np=2 u=4 th=512 pf={pf}", "rows", {"rows.sweep": 1, "rows.kl": 8, "rows.nv": 4, "rows.np": 2,
-                                                                    "rows.unroll": 4, "rows.threads": 512, "rows.prefetch": pf}))
-            v.append((f"sweep nv=4 np=1 u=4 th=512 pf={pf}", "rows", {"rows.sweep": 1, "rows.kl": 8, "rows.nv": 4, "rows.np": 1,
-                                                                    "rows.unroll": 4, "rows.threads": 512, "rows.prefetch": pf}))
     for items in (128, 256, 1024, 2048):
         v.append((f"merge items={items}", "merge", {"merge.items": items}))
     return v
@@ -159,18 +143,16 @@ def cfg2(args, emit, dev):
             for spec in args.tiles.split(","):
                 f = [int(x) for x in spec.split("x")]
                 T, BR = f[0], f[1]
-                kt = f[2] if len(f) > 2 else 0
-                thr = f[3] if len(f) > 3 else 0
-                depth = f[4] if len(f) > 4 else 0
-                ns_cap = f[5] if len(f) > 5 else 0
-                pool = f[6] if len(f) > 6 else 0
-                ksplit = f[7] if len(f) > 7 else 0
-                group = f[8] if len(f) > 8 else 0
+                thr = f[2] if len(f) > 2 else 0
+                depth = f[3] if len(f) > 3 else 0
+                ns_cap = f[4] if len(f) > 4 else 0
+                pool = f[5] if len(f) > 5 else 0
+                ksplit = f[6] if len(f) > 6 else 0
+                group = f[7] if len(f) > 7 else 0
 
-                def make(s, T=T, BR=BR, kt=kt, thr=thr, depth=depth, ns_cap=ns_cap, pool=pool, ksplit=ksplit, group=group):
+                def make(s, T=T, BR=BR, thr=thr, depth=depth, ns_cap=ns_cap, pool=pool, ksplit=ksplit, group=group):
                     A = spmm.DeviceCSR.from_host(host, dev.index)
                     _cabi.tune("reset", 0)
-                    _cabi.tune("tiled.kt", kt)
                     _cabi.tune("tiled.thr", thr)
                     _cabi.tune("tiled.depth", depth)
                     _cabi.tune("tiled.ns", ns_cap)
@@ -178,7 +160,8 @@ def cfg2(args, emit, dev):
                     _cabi.tune("tiled.ksplit", ksplit)
                     _cabi.tune("tiled.group", group)
                     try:
-                        A.build_tiles(T, BR)
+                        # cut for this k as AUTO cuts it; an explicit ksplit takes the form that reads tiled.ksplit (16-column k-tile)
+                        A.build_tiles(T, BR, 0 if ksplit else k)
                     finally:
                         _cabi.tune("reset", 0)
                     return A
@@ -192,15 +175,7 @@ def cfg2(args, emit, dev):
                     emit({"config": "cfg2", "k": k, "tiles": spec, "error": "no tile shape fits", "info": info})
                     continue
                 base = f"tiled {spec} T={info['rows_per_tile']} NS={info['window_slots']}"
-                vs = [(base, "tiled", {})]
-                if args.variants:
-                    vs += [(f"{base} ncw={ncw} u={u}", "tiled", {"tiled.ncw": ncw, "tiled.unroll": u})
-                           for ncw, u in ((8, 4), (8, 8), (12, 4), (12, 8), (16, 4), (16, 8), (20, 4), (24, 4))]
-                    vs += [(f"{base} ncw={ncw} u=4 npw=8", "tiled", {"tiled.ncw": ncw, "tiled.unroll": 4, "tiled.npw": 8})
-                           for ncw in (12, 16)]
-                if kt:
-                    vs = [(lab, kern, dict(tune, **{"tiled.kt": kt})) for lab, kern, tune in vs]  # launch with the k-tile the layout was cut for
-                run_variants("cfg2", sets, k, vs, args.iters, emit, host.nnz, n, {"tiles": info})
+                run_variants("cfg2", sets, k, [(base, "tiled", {})], args.iters, emit, host.nnz, n, {"tiles": info})
                 for A, _, _ in sets:
                     A.close()
                 del sets
@@ -415,7 +390,8 @@ def main():
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--variants", action="store_true")
     ap.add_argument("--cpu", action="store_true", help="also time the reference CPU code on cfg2")
-    ap.add_argument("--tiles", default="", help="cfg2: tile layouts to time, e.g. -1x16,64x16,32x8x32x2 (rows_per_tile x box_rows [x k-tile [x box threshold [x depth]]])")
+    ap.add_argument("--tiles", default="", help="cfg2: tile layouts to time, e.g. -1x16,64x16,32x8x2x3 (rows_per_tile x box_rows [x box threshold [x depth [x window slots "
+                    "[x pool rows [x ksplit [x group]]]]]]; the k-tile is the one AUTO cuts for k)")
     ap.add_argument("--only", default="", help="regex: run only the variants whose label matches")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "harness.jsonl"))
     args = ap.parse_args()

@@ -44,7 +44,7 @@ def main():
     ap.add_argument("--k", type=int, default=64)
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--sets", type=int, default=4)
-    ap.add_argument("--knobs", default=",tiled.prefetch=2")
+    ap.add_argument("--knobs", default="")
     ap.add_argument("--build", default="", help="build knobs, e.g. tiled.depth=3+tiled.group=2 (applied while the layouts are built)")
     ap.add_argument("--tile", default="-1x0", help="rows_per_tile x box_rows of the layout")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "probe_tiled.jsonl"))
