@@ -43,12 +43,14 @@ enum spmm_kernel
     SPMM_KERNEL_MERGE = 2, /* nnz-balanced merge-path with deterministic carry fix-up */
     /* ids 3, 4, 5 and 7 belonged to experimental layouts that never won a regime (profiles/r1_union.md); retired */
     SPMM_KERNEL_TILED = 6,    /* row tiles whose B rows are staged in shared memory by TMA (needs spmm_csr_build_tiles; even k) */
-    SPMM_KERNEL_STREAM = 8    /* k = 1, 2, 4, 8: CSR arrays streamed in nnz order, rows reduced from shared memory; bit-identical to the reference's mul-then-add (spmm_stream.cu) */
+    SPMM_KERNEL_STREAM = 8,   /* k = 1, 2, 4, 8: CSR arrays streamed in nnz order, rows reduced from shared memory; bit-identical to the reference's mul-then-add (spmm_stream.cu) */
+    SPMM_KERNEL_BSR = 9       /* b x b dense blocks: a team per block row loads each B row piece once for the b rows (needs spmm_csr_build_bsr; spmm_bsr.cu) */
 };
 
 const char *spmm_last_error(void);
 /* Name of the kernel family the calling thread's last multiply launched ("spmm_tiled_kernel", "spmm_rows_kernel",
- * "spmm_merge_kernel", "spmm_stream_kernel"; "" before the first launch): what AUTO chose, for measurement reports. */
+ * "spmm_merge_kernel", "spmm_stream_kernel", "spmm_bsr_kernel"; "" before the first launch): what AUTO chose, for
+ * measurement reports. */
 const char *spmm_last_kernel_name(void);
 int spmm_version(void);
 int spmm_device_count(int *count);
@@ -96,7 +98,9 @@ int spmm_csr_from_matrix_market(int device, const char *path, spmm_csr_t *out);
 int spmm_csr_destroy(spmm_csr_t A);
 int spmm_csr_info(spmm_csr_t A, int *n_rows, int *n_cols, long long *nnz, int *device);
 /* Writing through the returned value pointer requires spmm_csr_update_values_device(A, that pointer, stream) before the
- * next multiply: without it the tiled kernel uses the old values (its layout holds a copy of them). */
+ * next multiply: without it the tiled kernel uses the old values (its layout holds a copy of them). The BSR view reads
+ * d_vals itself and needs no refresh. A borrowed handle (copy=0) whose caller later changes the column ids keeps a stale
+ * tile layout and a stale BSR view: build them again (or drop them) after such a change. */
 int spmm_csr_device_ptrs(spmm_csr_t A, const int **d_rowptr, const int **d_colidx, const double **d_vals);
 /* New values for the same pattern: vals[nnz] in the handle's CSR order. The schedule, the CTA cuts and the tile
  * layout are kept; the values inside the tile layout are refreshed. Bits are copied (-0.0, NaN payloads survive).
@@ -132,6 +136,18 @@ int spmm_csr_build_tiles_for_k(spmm_csr_t A, int rows_per_tile, int box_rows, in
  * share of the non-zeros whose B row is staged on its own. Zeros when no layout is built. */
 int spmm_csr_tile_info(spmm_csr_t A, int *rows_per_tile, int *box_rows, int *window_slots, int *max_records,
                        double *reuse, double *single_fraction);
+/* b x b dense blocks (block sparse row) read straight from the CSR arrays: no copy, values are always the handle's d_vals.
+ * block_dim: 0 drops the view; 2..6 checks that the pattern is exactly b-blocked (else SPMM_ERR_UNSUPPORTED, message names
+ * the first block row that breaks it and why); -1 takes the largest b in 6..2 that fits (none: succeeds with *out_dim = 0).
+ * *out_dim (may be NULL) receives the block size in force.
+ * Exactly b-blocked: n_rows % b == 0; the b rows of block row R have one length L with L % b == 0; and for every q, t, i
+ * colidx[rowptr[R*b+i] + q*b + t] == c_q + t with c_q = colidx[rowptr[R*b] + q*b] and c_q % b == 0 (duplicates, missing
+ * entries and unaligned groups fail; empty block rows pass; columns need not be sorted: storage order is kept). Checked
+ * by one pass over the CSR on the device. A failed check leaves the view in force unchanged. With a view, AUTO takes
+ * SPMM_KERNEL_BSR in spmm_multiply_device / spmm_multiply_strided_device (and the host forms built on them) where it
+ * measured faster (DESIGN.md section 4.7) unless the schedule picked merge-path; the row-range, non-zero-range, window and
+ * scatter forms refuse SPMM_KERNEL_BSR with SPMM_ERR_UNSUPPORTED. */
+int spmm_csr_build_bsr(spmm_csr_t A, int block_dim, int *out_dim);
 /* Sub-matrix A[:, col_begin:col_end) with local column ids (column-block strategy,
  * north_star reading of sparseMatrixFatVectorMultiplyColumnWise). Built on the device. */
 int spmm_csr_column_block(spmm_csr_t A, int col_begin, int col_end, spmm_csr_t *out);

@@ -13,8 +13,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SPMM_B200_LIB") or os.path.join(HERE, "libspmm_b200.so")  # override: diagnostic builds only
 
 SPMM_OK, SPMM_ERR_INVALID, SPMM_ERR_CUDA, SPMM_ERR_NOMEM, SPMM_ERR_UNSUPPORTED = range(5)
-KERNEL_AUTO, KERNEL_ROWS, KERNEL_MERGE, KERNEL_TILED, KERNEL_STREAM = 0, 1, 2, 6, 8
-KERNELS = {"auto": KERNEL_AUTO, "rows": KERNEL_ROWS, "merge": KERNEL_MERGE, "tiled": KERNEL_TILED, "stream": KERNEL_STREAM}
+KERNEL_AUTO, KERNEL_ROWS, KERNEL_MERGE, KERNEL_TILED, KERNEL_STREAM, KERNEL_BSR = 0, 1, 2, 6, 8, 9
+KERNELS = {"auto": KERNEL_AUTO, "rows": KERNEL_ROWS, "merge": KERNEL_MERGE, "tiled": KERNEL_TILED, "stream": KERNEL_STREAM,
+           "bsr": KERNEL_BSR}
 
 
 class SpmmError(RuntimeError):
@@ -60,6 +61,7 @@ PROTOTYPES = {
     "spmm_csr_build_tiles": (_i, [_p, _i, _i]),
     "spmm_csr_build_tiles_for_k": (_i, [_p, _i, _i, _i]),
     "spmm_csr_column_span": (_i, [_p, _pi, _pi]),
+    "spmm_csr_build_bsr": (_i, [_p, _i, _pi]),
     "spmm_multiply_host_rows": (_i, [_p, _p, _i, _p, _i]),
     "spmm_multiply_host_sink": (_i, [_p, _p, _i, _p, _p, _i]),
     "spmm_fetch_c_sink": (_i, [_p, _p, _i, _i, _p, _p]),

@@ -195,6 +195,23 @@ int alloc_arrays(spmm_csr_s *A)
     return SPMM_OK;
 }
 
+// The BSR kernel computes whole block rows into a C of the matrix's shape; the partial forms (row ranges, non-zero ranges,
+// B windows, scatter) keep the CSR kernels, and the unknown ids they map to the row kernel do not include this one.
+static int refuse_bsr(int kernel, const char *form)
+{
+    if (kernel != SPMM_KERNEL_BSR)
+        return SPMM_OK;
+    set_error(std::string(form) + ": the BSR kernel serves spmm_multiply_device and spmm_multiply_strided_device only");
+    return SPMM_ERR_UNSUPPORTED;
+}
+
+// k range in which AUTO takes the BSR kernel on a handle with a view (DESIGN.md section 4.7, profiles/r3_bsr.md; B200,
+// 1000 W): at k = 128 it beat what AUTO runs without the view on fem_blocked b = 3 (254 against 295 us), b = 6 (299 against
+// 344 us) and the ten times larger b = 3 matrix (2.22 against 2.31 ms), and lost on b = 4 (292 against 248 us), where the
+// tile layout applies. Below k = 64 it lost on every matrix (2-11x at k <= 8: one block row per team is too little
+// parallel work per lane), and at k = 64 it lost on two of four.
+static bool bsr_auto_k(int k) { return k >= 128; }
+
 static int select_kernel(const spmm_csr_s *A, int kernel)
 {
     if (kernel == SPMM_KERNEL_AUTO)
@@ -474,8 +491,13 @@ int spmm_multiply_strided_device(spmm_csr_t A, const double *d_B, int ldb, doubl
     SPMM_CUDA(cudaSetDevice(A->device));
     cudaStream_t s = (cudaStream_t)stream;
     SPMM_REQUIRE(kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE ||
-                     kernel == SPMM_KERNEL_TILED || kernel == SPMM_KERNEL_STREAM,
+                     kernel == SPMM_KERNEL_TILED || kernel == SPMM_KERNEL_STREAM || kernel == SPMM_KERNEL_BSR,
                  "unknown kernel id");
+    if (kernel == SPMM_KERNEL_BSR)
+    {
+        SPMM_REQUIRE(A->bsr_b != 0, "BSR kernel requested but spmm_csr_build_bsr was not called (or found no block size)");
+        return launch_bsr(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
+    }
     if (kernel == SPMM_KERNEL_STREAM)
     {
         SPMM_REQUIRE(stream_shape_ok(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count),
@@ -491,6 +513,10 @@ int spmm_multiply_strided_device(spmm_csr_t A, const double *d_B, int ldb, doubl
         A->nnz >= tuning().stream_auto_min_nnz &&
         stream_shape_ok(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count))
         return launch_stream(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
+    // a handle with a BSR view, in the k range where its kernel was measured faster; the lazy tile layout is neither
+    // counted toward nor built by these launches
+    if (kernel == SPMM_KERNEL_AUTO && A->bsr_b != 0 && bsr_auto_k(k_count))
+        return launch_bsr(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
     if (kernel == SPMM_KERNEL_AUTO)
         auto_tile_layout(A, k_count);
     return launch_rows(A, 0, A->n_rows, 0, A->nnz, 0, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count,
@@ -502,6 +528,8 @@ int spmm_multiply_scatter_device(spmm_csr_t A, const double *d_B, int k, int n_d
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
+    if (int rc = refuse_bsr(kernel, "scatter multiply"))
+        return rc;
     SPMM_REQUIRE(n_dst >= 1 && n_dst <= 1 + SPMM_MAX_EXTRA, "n_dst must be between 1 and 8");
     SPMM_REQUIRE(d_C_list != nullptr, "d_C_list is NULL");
     SPMM_REQUIRE(kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE ||
@@ -543,6 +571,8 @@ int spmm_multiply_window_device(spmm_csr_t A, const double *d_B_window, int wind
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0 && window_first_row >= 0 && window_rows >= 0 && (long long)window_first_row + window_rows <= A->n_cols,
                  "window outside B");
+    if (int rc = refuse_bsr(kernel, "window multiply"))
+        return rc;
     if (A->n_rows == 0 || k == 0)
         return SPMM_OK;
     SPMM_REQUIRE(d_C != nullptr && (d_B_window != nullptr || A->nnz == 0), "d_B_window / d_C is NULL");
@@ -565,6 +595,8 @@ int spmm_multiply_rows_device(spmm_csr_t A, int row_begin, int row_end, const do
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
     SPMM_REQUIRE(0 <= row_begin && row_begin <= row_end && row_end <= A->n_rows, "row range outside the matrix");
+    if (int rc = refuse_bsr(kernel, "row-range multiply"))
+        return rc;
     if (row_begin == row_end || k == 0)
         return SPMM_OK;
     SPMM_REQUIRE(d_C_local != nullptr, "d_C_local is NULL");
@@ -628,6 +660,8 @@ int spmm_multiply_nnz_range_device(spmm_csr_t A, long long nnz_begin, long long 
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
     SPMM_REQUIRE(0 <= nnz_begin && nnz_begin <= nnz_end && nnz_end <= A->nnz, "non-zero range outside the matrix");
+    if (int rc = refuse_bsr(kernel, "non-zero-range multiply"))
+        return rc;
     if (nnz_begin == nnz_end || k == 0 || last_row < first_row)
         return SPMM_OK;
     SPMM_REQUIRE(0 <= first_row && last_row < A->n_rows, "row range outside the matrix");

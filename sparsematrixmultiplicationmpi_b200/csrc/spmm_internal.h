@@ -118,7 +118,8 @@ struct spmm_csr_s
     int *d_torder = nullptr;          // walking order of the tiles (nullptr: as they lie)
     int tl_stride = 0, tl_group = 0;  // detected far-band distance in rows, planes interleaved per super-group
     mutable bool tl_refreshed = false; // blob values rewritten since the last tiled launch (that launch is not programmatic)
-    // precomputed CTA cuts per (kind, grid size): kind 0 = rows of the CSR
+    int bsr_b = 0; // block size of the BSR view of the CSR arrays (spmm_bsr.cu), 0 = none
+    // precomputed CTA cuts per (kind, grid size): kind 0 = rows of the CSR, 3 = stream-kernel tiles, 9 = block rows of the BSR view
     mutable std::map<long long, int *> bounds;
     // merge-path scratch (carry rows), grown on demand; one set per handle, so merge multiplies enqueued on different streams
     // are ordered through carry_done (recorded after each fix-up) whenever the stream changes
@@ -151,6 +152,8 @@ int build_tiles(spmm_csr_s *A, int rows_per_tile, int box_rows, int kt_want, int
 // what AUTO cuts the tile layout for: 64-byte window rows for k <= 8; chunks shared by 2 / 4 CTAs (one k-tile group each) from k = 32 / 64
 inline int tiles_kt_for(int k) { return k <= 8 ? 8 : 16; }
 inline int tiles_ksplit_for(int k) { return k >= 64 ? 4 : (k >= 32 ? 2 : 1); }
+// BSR view (spmm_bsr.cu): A->bsr_b != 0; every (row, column) is one FMA chain in storage order, as in the CSR kernels
+int launch_bsr(const spmm_csr_s *A, const double *d_B, long long ldb, double *d_C, long long ldc, int kc, cudaStream_t stream);
 bool stream_shape_ok(const spmm_csr_s *A, const double *d_B, long long ldb, const double *d_C, long long ldc, int kc);
 int launch_stream(const spmm_csr_s *A, const double *d_B, long long ldb, double *d_C, long long ldc, int kc,
                   cudaStream_t stream);

@@ -99,6 +99,22 @@ def cop20k_A_shaped(n: int = 121_192, nnz: int = 2_624_331, seed: int = 20, nx: 
     return n, n, er[order].astype(np.int32), ec[order].astype(np.int32), vals[order], True
 
 
+def fem_blocked(dof: int, n_nodes: int, node_nnz: int, seed: int = 20):
+    """A FEM matrix with `dof` unknowns per mesh node: the node graph of cop20k_A_shaped(n_nodes, node_nnz, seed), every
+    node coupling expanded into a dense dof x dof block with values U[0.5, 1.5). Returns *general* records (the lower
+    triangle of the node graph mirrored here; symmetric records would be mirrored again inside the diagonal blocks).
+    Node sizes of cfg2's size: dof 3: 40,397 nodes, 291,592 entries; dof 4: 30,298, 164,020; dof 6: 20,199, 72,898."""
+    n, _, r, c, _, _ = cop20k_A_shaped(n=n_nodes, nnz=node_nnz, seed=seed)
+    off = r != c
+    nr = np.concatenate([r, c[off]]).astype(np.int64)
+    nc = np.concatenate([c, r[off]]).astype(np.int64)
+    i, j = np.meshgrid(np.arange(dof), np.arange(dof), indexing="ij")
+    rows = (nr[:, None] * dof + i.reshape(1, -1)).reshape(-1)
+    cols = (nc[:, None] * dof + j.reshape(1, -1)).reshape(-1)
+    vals = 0.5 + np.random.default_rng(seed + 1).random(rows.size)
+    return n * dof, n * dof, rows.astype(np.int32), cols.astype(np.int32), vals, False
+
+
 def expanded_nnz(rows, cols, symmetric: bool) -> int:
     return int(rows.size + (np.count_nonzero(rows != cols) if symmetric else 0))
 

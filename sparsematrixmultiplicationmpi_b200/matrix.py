@@ -144,6 +144,15 @@ class DeviceCSR:
         _cabi.check(_cabi.lib().spmm_csr_build_tiles_for_k(self.handle, rows_per_tile, box_rows, k))
         return self.tile_info()
 
+    def build_bsr(self, block_dim: int = -1) -> int:
+        """View the CSR as b x b dense blocks (spmm_csr_build_bsr, spmm_bsr.cu): no copy, the values stay the handle's.
+        block_dim: 2..6 checks that the pattern is exactly b-blocked (SpmmError with SPMM_ERR_UNSUPPORTED naming the first
+        block row that breaks it), -1 takes the largest b that fits, 0 drops the view. Returns the block size in force
+        (0: none). With a view, multiply(kernel="bsr") runs the BSR kernel and AUTO takes it where it measured faster."""
+        b = C.c_int()
+        _cabi.check(_cabi.lib().spmm_csr_build_bsr(self.handle, block_dim, C.byref(b)))
+        return b.value
+
     def tile_info(self) -> dict:
         t, b, ns, mr, r, sf = C.c_int(), C.c_int(), C.c_int(), C.c_int(), C.c_double(), C.c_double()
         _cabi.check(_cabi.lib().spmm_csr_tile_info(self.handle, C.byref(t), C.byref(b), C.byref(ns), C.byref(mr),
