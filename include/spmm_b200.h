@@ -157,26 +157,28 @@ int spmm_csr_column_span(spmm_csr_t A, int *min_col, int *max_col);
 
 /* ---- a3: sparseMatrixFatVectorMultiply (SparseMatrixFatVectorMultiply.cpp:11-31) ---- */
 
-/* C[n_rows x k] = A * B[n_cols x k], everything resident on the device. */
+/* C[n_rows x k] = A * B[n_cols x k], everything resident on the device.
+ * kernel: AUTO, ROWS, MERGE, TILED, STREAM or BSR; any other id is SPMM_ERR_INVALID. */
 int spmm_multiply_device(spmm_csr_t A, const double *d_B, int k, double *d_C, int kernel, void *stream);
 
 /* Row-wise strategy with the gather fused into the multiply (RowWise.cpp:36-50 + the MPI_Gatherv of :85-87,
  * or an all-gather): the C rows of this shard (n_rows x k, contiguous) are stored from registers to every one of
  * the n_dst (1..8) destinations — d_C_list[0] usually the local copy, the others peer GPUs' buffers mapped into
  * this process over NVLink (CUDA IPC / symmetric memory), each already offset to the shard's first row.
- * kernel: AUTO, ROWS, MERGE or TILED. No NCCL call, no staging copy; the caller synchronises the ranks
- * afterwards (a barrier) before anybody reads its buffer. */
+ * kernel: AUTO, ROWS, MERGE or TILED (BSR: SPMM_ERR_UNSUPPORTED, other ids: SPMM_ERR_INVALID). No NCCL call, no
+ * staging copy; the caller synchronises the ranks afterwards (a barrier) before anybody reads its buffer. */
 int spmm_multiply_scatter_device(spmm_csr_t A, const double *d_B, int k, int n_dst, double *const *d_C_list,
                                  int kernel, void *stream);
 
 /* Row-wise strategy without replicating B (RowWise.cpp:36-50 reads fatVector[colIndices[j]] only): d_B_window holds the
  * rows [window_first_row, window_first_row + window_rows) of B — the rows this shard's column ids name (see
- * spmm_csr_column_span), e.g. the rank's own rows plus a halo fetched from its neighbours. kernel: AUTO, ROWS or MERGE. */
+ * spmm_csr_column_span), e.g. the rank's own rows plus a halo fetched from its neighbours. kernel: AUTO, ROWS or MERGE (BSR:
+ * SPMM_ERR_UNSUPPORTED, other ids: SPMM_ERR_INVALID). */
 int spmm_multiply_window_device(spmm_csr_t A, const double *d_B_window, int window_first_row, int window_rows, int k,
                                 double *d_C, int kernel, void *stream);
 
 /* Strided form: B has leading dimension ldb, C has ldc; columns [k_begin, k_begin+k_count)
- * of B/C are computed (the k-slab split of ColumnWise.cpp:25-48). */
+ * of B/C are computed (the k-slab split of ColumnWise.cpp:25-48). kernel: as spmm_multiply_device. */
 int spmm_multiply_strided_device(spmm_csr_t A, const double *d_B, int ldb, double *d_C, int ldc,
                                  int k_begin, int k_count, int kernel, void *stream);
 
@@ -202,7 +204,8 @@ int spmm_host_threads(void); /* size of that host thread pool (env SPMM_HOST_THR
 void spmm_host_parallel_for(int n, void (*fn)(int, void *), void *ctx);
 
 /* ---- a4: row block [row_begin,row_end) (RowWise.cpp:26-50). d_C_local holds
- * (row_end-row_begin) x k, i.e. the rank's localResult before the Gatherv. ---- */
+ * (row_end-row_begin) x k, i.e. the rank's localResult before the Gatherv.
+ * kernel: AUTO, ROWS or MERGE as named, BSR SPMM_ERR_UNSUPPORTED, any other id runs the row kernel. ---- */
 int spmm_multiply_rows_device(spmm_csr_t A, int row_begin, int row_end, const double *d_B, int k,
                               double *d_C_local, int kernel, void *stream);
 
@@ -214,7 +217,7 @@ int spmm_multiply_rows_host(spmm_csr_t A, int row_begin, int row_end, const doub
  * (last_row-first_row+1) x k and receives, for each of those rows, the sum over
  * the range's elements only (boundary rows are therefore partial sums, to be
  * combined across ranks in rank order). Rows strictly inside get their full value;
- * empty rows inside get zeros. ---- */
+ * empty rows inside get zeros. kernel: as spmm_multiply_rows_device. ---- */
 int spmm_nnz_range_rows(spmm_csr_t A, long long nnz_begin, long long nnz_end, int *first_row, int *last_row);
 int spmm_multiply_nnz_range_device(spmm_csr_t A, long long nnz_begin, long long nnz_end, int first_row, int last_row,
                                    const double *d_B, int k, double *d_C_local, int kernel, void *stream);

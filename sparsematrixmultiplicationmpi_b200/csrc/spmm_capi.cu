@@ -1,8 +1,8 @@
 // spmm_capi.cu — the extern "C" boundary declared in include/spmm_b200.h.
 //
-// Thin by design: argument checks, device memory, the row-length schedule and
-// kernel selection. All arithmetic of the path lives in the CUDA kernels
-// (spmm_rows.cu, spmm_merge.cu, csr_build.cu); nothing here computes on the host.
+// Thin by design: argument checks, device memory and the row-length schedule; the kernel
+// is picked in spmm_dispatch.cu. All arithmetic of the path lives in the CUDA kernels
+// (spmm_kernels.cuh, spmm_tiled.cu, spmm_stream.cu, spmm_bsr.cu, csr_build.cu).
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -193,30 +193,6 @@ int alloc_arrays(spmm_csr_s *A)
     SPMM_CUDA(cudaMalloc(&A->d_vals, sizeof(double) * ((size_t)std::max<long long>(A->nnz, 1) + 8)));
     A->owns = true;
     return SPMM_OK;
-}
-
-// The BSR kernel computes whole block rows into a C of the matrix's shape; the partial forms (row ranges, non-zero ranges,
-// B windows, scatter) keep the CSR kernels, and the unknown ids they map to the row kernel do not include this one.
-static int refuse_bsr(int kernel, const char *form)
-{
-    if (kernel != SPMM_KERNEL_BSR)
-        return SPMM_OK;
-    set_error(std::string(form) + ": the BSR kernel serves spmm_multiply_device and spmm_multiply_strided_device only");
-    return SPMM_ERR_UNSUPPORTED;
-}
-
-// k range in which AUTO takes the BSR kernel on a handle with a view (DESIGN.md section 4.7, profiles/r3_bsr.md; B200,
-// 1000 W): at k = 128 it beat what AUTO runs without the view on fem_blocked b = 3 (254 against 295 us), b = 6 (299 against
-// 344 us) and the ten times larger b = 3 matrix (2.22 against 2.31 ms), and lost on b = 4 (292 against 248 us), where the
-// tile layout applies. Below k = 64 it lost on every matrix (2-11x at k <= 8: one block row per team is too little
-// parallel work per lane), and at k = 64 it lost on two of four.
-static bool bsr_auto_k(int k) { return k >= 128; }
-
-static int select_kernel(const spmm_csr_s *A, int kernel)
-{
-    if (kernel == SPMM_KERNEL_AUTO)
-        return A->sched.auto_kernel;
-    return kernel == SPMM_KERNEL_MERGE ? SPMM_KERNEL_MERGE : SPMM_KERNEL_ROWS;
 }
 
 } // namespace spmm
@@ -453,74 +429,20 @@ int spmm_csr_schedule(spmm_csr_t A, long long bins[8], int *max_row_len, double 
 
 // ---- multiply ---------------------------------------------------------------------
 
-// AUTO builds the tile layout the first time a multiply can use it (even k >= 4, mid-sized matrix with regular rows):
-// one-off, ~10 ms, about 10 bytes per non-zero next to the CSR; it is rebuilt when k moves to the other k-tile width (8 columns
-// for k <= 8) or to fewer k-tiles than CTAs share a chunk. spmm_tune_set("tiled", 0) or an explicit
-// spmm_csr_build_tiles(A, 0, 0) keeps the CSR kernels. Failure to build is not an error: the CSR kernels stay in charge.
-static void auto_tile_layout(spmm_csr_t A, int k)
-{
-    if (A->tl_auto && A->tl_T != 0 && (A->tl_ksplit > std::max(1, (k + 15) / 16) || (A->tl_kt == 8) != (k <= 8)))
-    {
-        free_tiles(A);
-        A->tl_tried = false;
-    }
-    if (A->tl_tried || A->tl_T != 0 || tuning().tiled == 0 || k < 4 || k % 2 != 0 || A->nnz < 200000 || A->nnz > (64ll << 20))
-        return;
-    // The layout costs about 150 multiplies to build: a handle that is multiplied once (the reference calls each function
-    // once per run, main.cpp:78) keeps the CSR row kernels; the layout is built when the handle comes back.
-    if (A->auto_calls++ < tuning().tiled_auto_after)
-        return;
-    A->tl_tried = true;
-    const int brc = build_tiles(A, -1, 0, tiles_kt_for(k), tuning().tiled_ksplit > 0 ? tuning().tiled_ksplit : tiles_ksplit_for(k));
-    A->tl_auto = true;
-    if (brc != SPMM_OK)
-        free_tiles(A);
-}
-
-
 int spmm_multiply_strided_device(spmm_csr_t A, const double *d_B, int ldb, double *d_C, int ldc, int k_begin,
                                  int k_count, int kernel, void *stream)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k_begin >= 0 && k_count >= 0, "negative column range");
     SPMM_REQUIRE(ldb >= k_begin + k_count && ldc >= k_begin + k_count, "leading dimension smaller than column range");
+    if (int rc = resolve_kernel(Form::whole, kernel, &kernel))
+        return rc;
     if (A->n_rows == 0 || k_count == 0)
         return SPMM_OK;
     SPMM_REQUIRE(d_C != nullptr, "d_C is NULL");
     SPMM_REQUIRE(d_B != nullptr || A->nnz == 0, "d_B is NULL");
-    SPMM_CUDA(cudaSetDevice(A->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    SPMM_REQUIRE(kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE ||
-                     kernel == SPMM_KERNEL_TILED || kernel == SPMM_KERNEL_STREAM || kernel == SPMM_KERNEL_BSR,
-                 "unknown kernel id");
-    if (kernel == SPMM_KERNEL_BSR)
-    {
-        SPMM_REQUIRE(A->bsr_b != 0, "BSR kernel requested but spmm_csr_build_bsr was not called (or found no block size)");
-        return launch_bsr(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
-    }
-    if (kernel == SPMM_KERNEL_STREAM)
-    {
-        SPMM_REQUIRE(stream_shape_ok(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count),
-                     "stream kernel: k must be 1, 2, 4 or 8 (B 16-byte aligned with an even leading dimension from k = 2), rows of at most 3072 / k non-zeros");
-        return launch_stream(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
-    }
-    SPMM_REQUIRE(kernel != SPMM_KERNEL_TILED || A->tl_T != 0, "tiled kernel requested but spmm_csr_build_tiles was not called (or found no fitting tile shape)");
-    if (select_kernel(A, kernel) == SPMM_KERNEL_MERGE)
-        return launch_merge(A, 0, A->n_rows, 0, A->nnz, 0, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
-    // k = 1 on matrices of 4 M non-zeros and more: streamed in nnz order (3.1 against 2.4 TB/s at 10.5 M non-zeros, and bit-identical to
-    // the reference); wider k / smaller matrices by spmm_tune_set("stream.kmax" / "stream.min_nnz") (profiles/r1_stream.md)
-    if (kernel == SPMM_KERNEL_AUTO && tuning().stream != 0 && k_count <= tuning().stream_auto_kmax &&
-        A->nnz >= tuning().stream_auto_min_nnz &&
-        stream_shape_ok(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count))
-        return launch_stream(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
-    // a handle with a BSR view, in the k range where its kernel was measured faster; the lazy tile layout is neither
-    // counted toward nor built by these launches
-    if (kernel == SPMM_KERNEL_AUTO && A->bsr_b != 0 && bsr_auto_k(k_count))
-        return launch_bsr(A, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, s);
-    if (kernel == SPMM_KERNEL_AUTO)
-        auto_tile_layout(A, k_count);
-    return launch_rows(A, 0, A->n_rows, 0, A->nnz, 0, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count,
-                       kernel == SPMM_KERNEL_ROWS ? 0 : (kernel == SPMM_KERNEL_AUTO ? 1 : kernel), s);
+    const Request r = {Form::whole, 0, A->n_rows, 0, A->nnz, 0, d_B + k_begin, ldb, d_C + k_begin, ldc, k_count, nullptr};
+    return multiply(A, r, kernel, (cudaStream_t)stream);
 }
 
 int spmm_multiply_scatter_device(spmm_csr_t A, const double *d_B, int k, int n_dst, double *const *d_C_list, int kernel,
@@ -528,13 +450,10 @@ int spmm_multiply_scatter_device(spmm_csr_t A, const double *d_B, int k, int n_d
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
-    if (int rc = refuse_bsr(kernel, "scatter multiply"))
+    if (int rc = resolve_kernel(Form::scatter, kernel, &kernel))
         return rc;
     SPMM_REQUIRE(n_dst >= 1 && n_dst <= 1 + SPMM_MAX_EXTRA, "n_dst must be between 1 and 8");
     SPMM_REQUIRE(d_C_list != nullptr, "d_C_list is NULL");
-    SPMM_REQUIRE(kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE ||
-                     kernel == SPMM_KERNEL_TILED,
-                 "scatter multiply: kernel must be auto, rows, merge or tiled");
     if (A->n_rows == 0 || k == 0)
         return SPMM_OK;
     ExtraDst x;
@@ -547,16 +466,8 @@ int spmm_multiply_scatter_device(spmm_csr_t A, const double *d_B, int k, int n_d
             x.off[x.n++] = (long long)(((intptr_t)d_C_list[i] - (intptr_t)d_C_list[0]) / (intptr_t)sizeof(double));
     }
     SPMM_REQUIRE(d_B != nullptr || A->nnz == 0, "d_B is NULL");
-    SPMM_REQUIRE(kernel != SPMM_KERNEL_TILED || A->tl_T != 0, "tiled kernel requested but spmm_csr_build_tiles was not called");
-    SPMM_CUDA(cudaSetDevice(A->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    double *d_C = d_C_list[0];
-    if (select_kernel(A, kernel) == SPMM_KERNEL_MERGE)
-        return launch_merge(A, 0, A->n_rows, 0, A->nnz, 0, d_B, k, d_C, k, k, s, &x);
-    if (kernel == SPMM_KERNEL_AUTO)
-        auto_tile_layout(A, k);
-    return launch_rows(A, 0, A->n_rows, 0, A->nnz, 0, d_B, k, d_C, k, k,
-                       kernel == SPMM_KERNEL_ROWS ? 0 : (kernel == SPMM_KERNEL_AUTO ? 1 : kernel), s, &x);
+    const Request r = {Form::scatter, 0, A->n_rows, 0, A->nnz, 0, d_B, k, d_C_list[0], k, k, &x};
+    return multiply(A, r, kernel, (cudaStream_t)stream);
 }
 
 int spmm_multiply_device(spmm_csr_t A, const double *d_B, int k, double *d_C, int kernel, void *stream)
@@ -571,22 +482,15 @@ int spmm_multiply_window_device(spmm_csr_t A, const double *d_B_window, int wind
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0 && window_first_row >= 0 && window_rows >= 0 && (long long)window_first_row + window_rows <= A->n_cols,
                  "window outside B");
-    if (int rc = refuse_bsr(kernel, "window multiply"))
+    if (int rc = resolve_kernel(Form::window, kernel, &kernel))
         return rc;
     if (A->n_rows == 0 || k == 0)
         return SPMM_OK;
     SPMM_REQUIRE(d_C != nullptr && (d_B_window != nullptr || A->nnz == 0), "d_B_window / d_C is NULL");
-    SPMM_REQUIRE(kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE,
-                 "window multiply: kernel must be auto, rows or merge (the CSR kernels read B rows one by one)");
-    SPMM_CUDA(cudaSetDevice(A->device));
     // virtual base: row j of B sits at d_B_window + (j - window_first_row) * k; only rows named by column ids are read
     const double *base = d_B_window - (long long)window_first_row * k;
-    if (select_kernel(A, kernel) == SPMM_KERNEL_MERGE)
-        return launch_merge(A, 0, A->n_rows, 0, A->nnz, 0, base, k, d_C, k, k, (cudaStream_t)stream);
-    set_b_window(true);
-    const int rc = launch_rows(A, 0, A->n_rows, 0, A->nnz, 0, base, k, d_C, k, k, 0, (cudaStream_t)stream);
-    set_b_window(false);
-    return rc;
+    const Request r = {Form::window, 0, A->n_rows, 0, A->nnz, 0, base, k, d_C, k, k, nullptr};
+    return multiply(A, r, kernel, (cudaStream_t)stream);
 }
 
 int spmm_multiply_rows_device(spmm_csr_t A, int row_begin, int row_end, const double *d_B, int k,
@@ -595,17 +499,14 @@ int spmm_multiply_rows_device(spmm_csr_t A, int row_begin, int row_end, const do
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
     SPMM_REQUIRE(0 <= row_begin && row_begin <= row_end && row_end <= A->n_rows, "row range outside the matrix");
-    if (int rc = refuse_bsr(kernel, "row-range multiply"))
+    if (int rc = resolve_kernel(Form::rows, kernel, &kernel))
         return rc;
     if (row_begin == row_end || k == 0)
         return SPMM_OK;
     SPMM_REQUIRE(d_C_local != nullptr, "d_C_local is NULL");
-    SPMM_CUDA(cudaSetDevice(A->device));
     SPMM_REQUIRE(d_B != nullptr || A->nnz == 0, "d_B is NULL");
-    if (select_kernel(A, kernel) == SPMM_KERNEL_MERGE)
-        return launch_merge(A, row_begin, row_end, 0, A->nnz, row_begin, d_B, k, d_C_local, k, k, (cudaStream_t)stream);
-    return launch_rows(A, row_begin, row_end, 0, A->nnz, row_begin, d_B, k, d_C_local, k, k, 0,
-                       (cudaStream_t)stream);
+    const Request r = {Form::rows, row_begin, row_end, 0, A->nnz, row_begin, d_B, k, d_C_local, k, k, nullptr};
+    return multiply(A, r, kernel, (cudaStream_t)stream);
 }
 
 // Rows touched by a non-zero range: first = the row holding element nnz_begin,
@@ -660,18 +561,14 @@ int spmm_multiply_nnz_range_device(spmm_csr_t A, long long nnz_begin, long long 
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
     SPMM_REQUIRE(k >= 0, "k is negative");
     SPMM_REQUIRE(0 <= nnz_begin && nnz_begin <= nnz_end && nnz_end <= A->nnz, "non-zero range outside the matrix");
-    if (int rc = refuse_bsr(kernel, "non-zero-range multiply"))
+    if (int rc = resolve_kernel(Form::nnz_range, kernel, &kernel))
         return rc;
     if (nnz_begin == nnz_end || k == 0 || last_row < first_row)
         return SPMM_OK;
     SPMM_REQUIRE(0 <= first_row && last_row < A->n_rows, "row range outside the matrix");
     SPMM_REQUIRE(d_C_local != nullptr && d_B != nullptr, "d_B/d_C_local is NULL");
-    SPMM_CUDA(cudaSetDevice(A->device));
-    if (select_kernel(A, kernel) == SPMM_KERNEL_MERGE)
-        return launch_merge(A, first_row, last_row + 1, nnz_begin, nnz_end, first_row, d_B, k, d_C_local, k, k,
-                            (cudaStream_t)stream);
-    return launch_rows(A, first_row, last_row + 1, nnz_begin, nnz_end, first_row, d_B, k, d_C_local, k, k, 0,
-                       (cudaStream_t)stream);
+    const Request r = {Form::nnz_range, first_row, last_row + 1, nnz_begin, nnz_end, first_row, d_B, k, d_C_local, k, k, nullptr};
+    return multiply(A, r, kernel, (cudaStream_t)stream);
 }
 
 } // extern "C"

@@ -70,40 +70,109 @@ Shape pick_shape(const double *d_B, long long ldb, const double *d_C, long long 
     s.tiles = (kq + tile - 1) / tile;
     return s;
 }
+
+// the fields every CSR kernel reads
+SpmmArgs csr_args(const spmm_csr_s *A, const Request &r)
+{
+    SpmmArgs args = {};
+    if (r.extra)
+        args.extra = *r.extra;
+    args.rowptr = A->d_rowptr;
+    args.colidx = A->d_colidx;
+    args.vals = A->d_vals;
+    args.B = r.B;
+    args.C = r.C;
+    args.ldb = r.ldb;
+    args.ldc = r.ldc;
+    args.row_begin = r.row_begin;
+    args.row_end = r.row_end;
+    args.nnz_lo = (int)r.nnz_lo;
+    args.nnz_hi = (int)r.nnz_hi;
+    args.c_row0 = r.c_row0;
+    args.kc = r.kc;
+    return args;
+}
+
+// k range in which AUTO takes the BSR kernel on a handle with a view (DESIGN.md section 4.7, profiles/r3_bsr.md; B200,
+// 1000 W): at k = 128 it beat what AUTO runs without the view on fem_blocked b = 3 (254 against 295 us), b = 6 (299 against
+// 344 us) and the ten times larger b = 3 matrix (2.22 against 2.31 ms), and lost on b = 4 (292 against 248 us), where the
+// tile layout applies. Below k = 64 it lost on every matrix (2-11x at k <= 8: one block row per team is too little
+// parallel work per lane), and at k = 64 it lost on two of four.
+bool bsr_auto_k(int k) { return k >= 128; }
 } // namespace
 
-// set around a launch whose B pointer is the virtual base of a window of rows (rows outside the window are not mapped):
-// nothing may touch B beyond the rows the matrix's column ids name — no bulk prefetch of "all of B"
-static thread_local bool t_b_is_window = false;
-void set_b_window(bool on) { t_b_is_window = on; }
-
-int launch_rows(const spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, long long nnz_hi, int c_row0,
-                const double *d_B, long long ldb, double *d_C, long long ldc, int kc, int derived,
-                cudaStream_t stream, const ExtraDst *extra)
+int resolve_kernel(Form form, int kernel, int *effective)
 {
-    if (row_end <= row_begin || kc <= 0)
-        return SPMM_OK;
-    const Tuning &t = tuning();
-    const Shape s = pick_shape(d_B, ldb, d_C, ldc, kc);
-    // whole-matrix launch with a derived layout on the handle: use it when the shape fits
-    const bool whole = row_begin == 0 && row_end == A->n_rows && nnz_lo == 0 && nnz_hi == A->nnz && c_row0 == 0;
-    if (derived && whole)
+    *effective = kernel;
+    // The BSR kernel computes whole block rows into a C of the matrix's shape; the partial forms keep the CSR kernels.
+    if (kernel == SPMM_KERNEL_BSR && form != Form::whole)
     {
-        if (derived == 6 || (derived == 1 && A->tl_T && t.tiled != 0))
-        {
-            // tile layout: measured faster than the CSR kernels from k = 8 up when rows of a tile share B rows (profiles/r1_tiled.md)
-            const bool fits = tiled_shape_ok(A, d_B, ldb, d_C, ldc, kc);
-            const double staged = (double)A->tl_box_rows_loaded + (double)A->tl_single_rows;
-            const double reuse = staged > 0 ? (double)A->nnz / staged : 0.0;
-            if (fits && (derived == 6 || t.tiled == 1 || (kc >= (A->tl_kt == 8 ? 4 : 8) && reuse >= 2.0 && A->tl_drains * 20 <= A->tl_tiles)))
-                return launch_tiled(A, d_B, ldb, d_C, ldc, kc, stream, extra);
-            if (derived == 6)
-            {
-                set_error("tiled kernel: needs even k, even leading dimensions and 16-byte aligned B and C");
-                return SPMM_ERR_UNSUPPORTED;
-            }
-        }
+        set_error("the BSR kernel serves spmm_multiply_device and spmm_multiply_strided_device only");
+        return SPMM_ERR_UNSUPPORTED;
     }
+    if (kernel == SPMM_KERNEL_AUTO || kernel == SPMM_KERNEL_ROWS || kernel == SPMM_KERNEL_MERGE || kernel == SPMM_KERNEL_BSR)
+        return SPMM_OK;
+    // the row-range and non-zero-range forms run the row kernel for every other id
+    if (form == Form::rows || form == Form::nnz_range)
+    {
+        *effective = SPMM_KERNEL_ROWS;
+        return SPMM_OK;
+    }
+    // the tiled kernel stages B rows by TMA boxes (not only the rows a window holds); the stream kernel writes whole rows of one C
+    SPMM_REQUIRE(kernel == SPMM_KERNEL_TILED ? form != Form::window : kernel == SPMM_KERNEL_STREAM && form == Form::whole,
+                 "kernel id not served by this multiply form (include/spmm_b200.h lists the ids of each)");
+    return SPMM_OK;
+}
+
+// AUTO: merge-path where the schedule picked it; then, for the whole-matrix forms, the stream kernel and the BSR view; then,
+// with the scatter form too, the tile layout (built lazily); else the row kernel
+static int auto_kernel(spmm_csr_s *A, const Request &r)
+{
+    if (A->sched.auto_kernel == SPMM_KERNEL_MERGE)
+        return SPMM_KERNEL_MERGE;
+    // k = 1 on matrices of 4 M non-zeros and more: streamed in nnz order (3.1 against 2.4 TB/s at 10.5 M non-zeros, and
+    // bit-identical to the reference); wider k / smaller matrices by spmm_tune_set("stream.kmax" / "stream.min_nnz")
+    // (profiles/r1_stream.md)
+    const Tuning &t = tuning();
+    if (r.form == Form::whole && t.stream != 0 && r.kc <= t.stream_auto_kmax && A->nnz >= t.stream_auto_min_nnz &&
+        stream_shape_ok(A, r.B, r.ldb, r.C, r.ldc, r.kc))
+        return SPMM_KERNEL_STREAM;
+    // a handle with a BSR view, in the k range where its kernel was measured faster; the lazy tile layout is neither
+    // counted toward nor built by these launches
+    if (r.form == Form::whole && A->bsr_b != 0 && bsr_auto_k(r.kc))
+        return SPMM_KERNEL_BSR;
+    if (r.form != Form::whole && r.form != Form::scatter)
+        return SPMM_KERNEL_ROWS;
+    auto_tile_layout(A, r.kc);
+    return tiled_auto_ok(A, r) ? SPMM_KERNEL_TILED : SPMM_KERNEL_ROWS;
+}
+
+int multiply(spmm_csr_s *A, const Request &r, int kernel, cudaStream_t stream)
+{
+    SPMM_CUDA(cudaSetDevice(A->device));
+    // what an explicit request needs from the handle is checked at launch time
+    if (kernel == SPMM_KERNEL_BSR)
+        SPMM_REQUIRE(A->bsr_b != 0, "BSR kernel requested but spmm_csr_build_bsr was not called (or found no block size)");
+    if (kernel == SPMM_KERNEL_STREAM)
+        SPMM_REQUIRE(stream_shape_ok(A, r.B, r.ldb, r.C, r.ldc, r.kc),
+                     "stream kernel: k must be 1, 2, 4 or 8 (B 16-byte aligned with an even leading dimension from k = 2), rows of at most 3072 / k non-zeros");
+    if (kernel == SPMM_KERNEL_TILED)
+        if (int rc = tiled_check(A, r))
+            return rc;
+    switch (kernel == SPMM_KERNEL_AUTO ? auto_kernel(A, r) : kernel)
+    {
+    case SPMM_KERNEL_MERGE: return launch_merge(A, r, stream);
+    case SPMM_KERNEL_TILED: return launch_tiled(A, r, stream);
+    case SPMM_KERNEL_STREAM: return launch_stream(A, r.B, r.ldb, r.C, r.ldc, r.kc, stream);
+    case SPMM_KERNEL_BSR: return launch_bsr(A, r.B, r.ldb, r.C, r.ldc, r.kc, stream);
+    default: return launch_rows(A, r, stream);
+    }
+}
+
+int launch_rows(const spmm_csr_s *A, const Request &r, cudaStream_t stream)
+{
+    const Tuning &t = tuning();
+    const Shape s = pick_shape(r.B, r.ldb, r.C, r.ldc, r.kc);
     int np = 1;
     if (s.nv == 1)
     {
@@ -120,54 +189,36 @@ int launch_rows(const spmm_csr_s *A, int row_begin, int row_end, long long nnz_l
     np = std::max(1, std::min(np, 32 / s.kl));
     // B larger than L2 (gathers go to HBM): more rows in flight per team pay (cfg5: 25.5 -> 23.6 ms at unroll 4); B resident
     // in L2 / L1 (cfg2): 2 is the measured optimum for wide pieces
-    const bool b_beyond_l2 = (long long)A->n_cols * kc * 8 > device_props(A->device).l2_bytes;
+    const bool b_beyond_l2 = (long long)A->n_cols * r.kc * 8 > device_props(A->device).l2_bytes;
     int u = t.rows_unroll > 0 ? t.rows_unroll : (np >= 8 ? 1 : np >= 2 ? 2 : (s.nv >= 4 ? (b_beyond_l2 ? 4 : 2) : 4));
 
-    SpmmArgs args = {};
-    if (extra)
-        args.extra = *extra;
-    args.rowptr = A->d_rowptr;
-    args.colidx = A->d_colidx;
-    args.vals = A->d_vals;
-    args.B = d_B;
-    args.C = d_C;
-    args.ldb = ldb;
-    args.ldc = ldc;
-    args.row_begin = row_begin;
-    args.row_end = row_end;
-    args.nnz_lo = (int)nnz_lo;
-    args.nnz_hi = (int)nnz_hi;
-    args.c_row0 = c_row0;
-    args.kc = kc;
+    SpmmArgs args = csr_args(A, r);
     // L2 prefetch only when the operands are 16-byte aligned, B is one contiguous block that starts
     // at column 0 of its rows (no k-slab), and the A arrays are the handle's own (padded) allocations
-    const bool aligned = ((uintptr_t)A->d_colidx % 16 == 0) && ((uintptr_t)A->d_vals % 16 == 0) && ((uintptr_t)d_B % 16 == 0);
+    const bool aligned = ((uintptr_t)A->d_colidx % 16 == 0) && ((uintptr_t)A->d_vals % 16 == 0) && ((uintptr_t)r.B % 16 == 0);
     args.prefetch = aligned ? (t.rows_prefetch >= 0 ? t.rows_prefetch : 3) : 0;
-    args.b_bytes = (ldb == kc && !t_b_is_window) ? (long long)A->n_cols * ldb * 8 : 0;
+    // a window of B rows: nothing beyond the rows the column ids name may be touched (no prefetch of "all of B")
+    args.b_bytes = (r.ldb == r.kc && r.form != Form::window) ? (long long)A->n_cols * r.ldb * 8 : 0;
     note_kernel("spmm_rows_kernel");
     return s.w == 2 ? launch_rows_w2(A, s.kl, s.nv, np, u, args, s.tiles, A->device, stream)
                     : launch_rows_w1(A, s.kl, s.nv, np, u, args, s.tiles, A->device, stream);
 }
 
-int launch_merge(spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, long long nnz_hi, int c_row0,
-                 const double *d_B, long long ldb, double *d_C, long long ldc, int kc, cudaStream_t stream,
-                 const ExtraDst *extra)
+int launch_merge(spmm_csr_s *A, const Request &r, cudaStream_t stream)
 {
-    if (row_end <= row_begin || kc <= 0)
-        return SPMM_OK;
     const Tuning &t = tuning();
-    Shape s = pick_shape(d_B, ldb, d_C, ldc, kc);
+    Shape s = pick_shape(r.B, r.ldb, r.C, r.ldc, r.kc);
     // Team shape: pick_shape's (8 lanes x 2 accesses at k = 32). Measured on cfg3 (R-MAT 2^22, k = 32) after the kernel was
     // rebuilt around batches of KL non-zeros (coalesced id/value loads one batch ahead, B rows gathered 4 at a time whatever
     // rows they belong to): 8 x 2 unroll 4 at 80 registers 2.17 ms, 16 x 1 2.34 ms, unroll 8 (127 registers) 4.5 ms
     // (gpurun_out/s5_tune_mb1.jsonl); the row-by-row kernel before it took 3.06-3.50 ms.
     const int u = t.rows_unroll > 0 ? t.rows_unroll : (s.nv >= 4 ? 2 : 4);
-    const long long total = (long long)(row_end - row_begin) + (nnz_hi - nnz_lo);
+    const long long total = (long long)(r.row_end - r.row_begin) + (r.nnz_hi - r.nnz_lo);
     long long items = t.merge_items > 0 ? t.merge_items : 512;
     // enough teams to fill the machine, few enough that the carry rows stay a small fraction of C
     // (a shard of long rows — the first non-zero range of an R-MAT matrix averages 477 per row — is cut less finely: every
     // team inside a row leaves a carry slot and the fix-up walks them in order; measured per range in gpurun_out/s28_*)
-    const double avg_row = (double)(nnz_hi - nnz_lo) / std::max(1, row_end - row_begin);
+    const double avg_row = (double)(r.nnz_hi - r.nnz_lo) / std::max(1, r.row_end - r.row_begin);
     const int wave = t.merge_wave > 0 ? t.merge_wave : (avg_row > 256.0 ? 32 : 64);
     const long long teams_per_wave = (long long)device_props(A->device).sm_count * wave * (32 / s.kl);
     while (items > 64 && (total + items - 1) / items < teams_per_wave)
@@ -196,22 +247,7 @@ int launch_merge(spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, lo
         A->carry_rows = (size_t)(2 * n_teams);
     }
 
-    SpmmArgs args = {};
-    if (extra)
-        args.extra = *extra;
-    args.rowptr = A->d_rowptr;
-    args.colidx = A->d_colidx;
-    args.vals = A->d_vals;
-    args.B = d_B;
-    args.C = d_C;
-    args.ldb = ldb;
-    args.ldc = ldc;
-    args.row_begin = row_begin;
-    args.row_end = row_end;
-    args.nnz_lo = (int)nnz_lo;
-    args.nnz_hi = (int)nnz_hi;
-    args.c_row0 = c_row0;
-    args.kc = kc;
+    SpmmArgs args = csr_args(A, r);
     args.items_per_team = (int)items;
     args.n_teams = (int)n_teams;
     args.carry = A->d_carry;

@@ -132,18 +132,39 @@ struct spmm_csr_s
 
 namespace spmm
 {
+// The device multiply forms: the whole matrix (spmm_multiply_device, _strided_device), scatter, a window of B rows (nothing
+// beyond them may be read), a row range and a non-zero range; each accepts its own kernel ids (DESIGN.md section 4.3)
+enum class Form { whole, scatter, window, rows, nnz_range };
+
+// One device multiply: rows [row_begin,row_end), each clipped to the non-zero range [nnz_lo,nnz_hi); row c_row0 is
+// stored at C[0]; kc columns of B and C
+struct Request
+{
+    Form form;
+    int row_begin, row_end;
+    long long nnz_lo, nnz_hi;
+    int c_row0;
+    const double *B;
+    long long ldb;
+    double *C;
+    long long ldc;
+    int kc;
+    const struct ExtraDst *extra; // scatter: the further copies of C (nullptr: none)
+};
+
+// The kernel `form` runs for the id `kernel` (AUTO stays AUTO), or the status that refuses the id (spmm_dispatch.cu)
+int resolve_kernel(Form form, int kernel, int *effective);
+// The one place that picks the kernel for a request; `kernel` as resolve_kernel returned it for req.form
+int multiply(spmm_csr_s *A, const Request &req, int kernel, cudaStream_t stream);
+
 // launchers implemented in the kernel translation units
-// rows [row_begin,row_end), each clipped to the non-zero range [nnz_lo,nnz_hi); row c_row0 is stored at d_C[0]
-int launch_rows(const spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, long long nnz_hi, int c_row0,
-                const double *d_B, long long ldb, double *d_C, long long ldc, int kc, int derived,
-                cudaStream_t stream, const struct ExtraDst *extra = nullptr); // derived: 0 CSR row kernel only, 1 best available, 6 tiled
-void set_b_window(bool on); // the next launch_rows of this thread gets a window of B rows (no whole-B prefetch)
-int launch_merge(spmm_csr_s *A, int row_begin, int row_end, long long nnz_lo, long long nnz_hi, int c_row0,
-                 const double *d_B, long long ldb, double *d_C, long long ldc, int kc, cudaStream_t stream,
-                 const struct ExtraDst *extra = nullptr);
-bool tiled_shape_ok(const spmm_csr_s *A, const double *d_B, long long ldb, const double *d_C, long long ldc, int kc);
-int launch_tiled(const spmm_csr_s *A, const double *d_B, long long ldb, double *d_C, long long ldc, int kc,
-                 cudaStream_t stream, const struct ExtraDst *extra = nullptr);
+int launch_rows(const spmm_csr_s *A, const Request &req, cudaStream_t stream);
+int launch_merge(spmm_csr_s *A, const Request &req, cudaStream_t stream);
+// tile layout (spmm_tiled.cu): what an explicit TILED request needs (status), when AUTO builds the layout, when AUTO uses it
+int tiled_check(const spmm_csr_s *A, const Request &req);
+void auto_tile_layout(spmm_csr_s *A, int k);
+bool tiled_auto_ok(const spmm_csr_s *A, const Request &req);
+int launch_tiled(const spmm_csr_s *A, const Request &req, cudaStream_t stream);
 void free_tiles(spmm_csr_s *A);
 // new values (d_src[nnz], CSR order, on A's device) into A->d_vals (skipped when d_src is A->d_vals) and into the value
 // streams of the tile layout, enqueued on `stream`; the schedule, the CTA cuts and the rest of the layout are kept

@@ -1428,21 +1428,64 @@ void free_tiles(spmm_csr_s *A)
     A->tl_box_rows_loaded = A->tl_single_rows = 0;
 }
 
-bool tiled_shape_ok(const spmm_csr_s *A, const double *d_B, long long ldb, const double *d_C, long long ldc, int kc)
+static bool tiled_shape_ok(const spmm_csr_s *A, const Request &r)
 {
-    return A->tl_T > 0 && kc >= 2 && kc % 2 == 0 && ldb % 2 == 0 && ldc % 2 == 0 && ((uintptr_t)d_B % 16 == 0) &&
-           ((uintptr_t)d_C % 16 == 0) && (unsigned long long)ldb * 8ull < (1ull << 40);
+    return A->tl_T > 0 && r.kc >= 2 && r.kc % 2 == 0 && r.ldb % 2 == 0 && r.ldc % 2 == 0 && ((uintptr_t)r.B % 16 == 0) &&
+           ((uintptr_t)r.C % 16 == 0) && (unsigned long long)r.ldb * 8ull < (1ull << 40);
 }
 
-int launch_tiled(const spmm_csr_s *A, const double *d_B, long long ldb, double *d_C, long long ldc, int kc,
-                 cudaStream_t stream, const ExtraDst *extra)
+int tiled_check(const spmm_csr_s *A, const Request &r)
 {
-    const ExtraDst x = extra ? *extra : ExtraDst();
+    SPMM_REQUIRE(A->tl_T != 0, "tiled kernel requested but spmm_csr_build_tiles was not called (or found no fitting tile shape)");
+    if (tiled_shape_ok(A, r))
+        return SPMM_OK;
+    set_error("tiled kernel: needs even k, even leading dimensions and 16-byte aligned B and C");
+    return SPMM_ERR_UNSUPPORTED;
+}
+
+// AUTO builds the tile layout the first time a multiply can use it (even k >= 4, mid-sized matrix with regular rows):
+// one-off, ~10 ms, about 10 bytes per non-zero next to the CSR; it is rebuilt when k moves to the other k-tile width (8 columns
+// for k <= 8) or to fewer k-tiles than CTAs share a chunk. spmm_tune_set("tiled", 0) or an explicit
+// spmm_csr_build_tiles(A, 0, 0) keeps the CSR kernels. Failure to build is not an error: the CSR kernels stay in charge.
+void auto_tile_layout(spmm_csr_s *A, int k)
+{
+    if (A->tl_auto && A->tl_T != 0 && (A->tl_ksplit > std::max(1, (k + 15) / 16) || (A->tl_kt == 8) != (k <= 8)))
+    {
+        free_tiles(A);
+        A->tl_tried = false;
+    }
+    if (A->tl_tried || A->tl_T != 0 || tuning().tiled == 0 || k < 4 || k % 2 != 0 || A->nnz < 200000 || A->nnz > (64ll << 20))
+        return;
+    // The layout costs about 150 multiplies to build: a handle that is multiplied once (the reference calls each function
+    // once per run, main.cpp:78) keeps the CSR row kernels; the layout is built when the handle comes back.
+    if (A->auto_calls++ < tuning().tiled_auto_after)
+        return;
+    A->tl_tried = true;
+    const int brc = build_tiles(A, -1, 0, tiles_kt_for(k), tuning().tiled_ksplit > 0 ? tuning().tiled_ksplit : tiles_ksplit_for(k));
+    A->tl_auto = true;
+    if (brc != SPMM_OK)
+        free_tiles(A);
+}
+
+// tile layout: measured faster than the CSR kernels from k = 8 up when rows of a tile share B rows (profiles/r1_tiled.md)
+bool tiled_auto_ok(const spmm_csr_s *A, const Request &r)
+{
+    const Tuning &t = tuning();
+    if (t.tiled == 0 || !tiled_shape_ok(A, r))
+        return false;
+    const double staged = (double)A->tl_box_rows_loaded + (double)A->tl_single_rows;
+    const double reuse = staged > 0 ? (double)A->nnz / staged : 0.0;
+    return t.tiled == 1 || (r.kc >= (A->tl_kt == 8 ? 4 : 8) && reuse >= 2.0 && A->tl_drains * 20 <= A->tl_tiles);
+}
+
+int launch_tiled(const spmm_csr_s *A, const Request &r, cudaStream_t stream)
+{
+    const ExtraDst x = r.extra ? *r.extra : ExtraDst();
     note_kernel("spmm_tiled_kernel");
     // the kernel's shape is the one the layout was cut for
     if (A->tl_kt == 8)
-        return launch_tiled_t<8, 16, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
-    return launch_tiled_t<16, 16, 4, 4>(A, d_B, ldb, d_C, ldc, kc, stream, x);
+        return launch_tiled_t<8, 16, 4, 4>(A, r.B, r.ldb, r.C, r.ldc, r.kc, stream, x);
+    return launch_tiled_t<16, 16, 4, 4>(A, r.B, r.ldb, r.C, r.ldc, r.kc, stream, x);
 }
 
 int update_values(spmm_csr_s *A, const double *d_src, cudaStream_t stream)

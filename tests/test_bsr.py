@@ -17,7 +17,7 @@ from conftest import REL_TOL, assert_close_rel
 gpu = pytest.mark.gpu
 KEEP_NAN = np.array([0x7FF80000DEADBEEF], dtype=np.uint64).view(np.float64)[0]
 
-# k values for which AUTO takes the BSR kernel on a handle with a view (spmm_capi.cu, bsr_auto_k; profiles/r3_bsr.md)
+# k values for which AUTO takes the BSR kernel on a handle with a view (spmm_dispatch.cu, bsr_auto_k; profiles/r3_bsr.md)
 def AUTO_BSR_KS(k):
     return k >= 128
 
