@@ -71,6 +71,35 @@ int spmm_csr_create_device(int device, int n_rows, int n_cols, long long nnz,
                            const int *d_rowptr, const int *d_colidx, const double *d_vals,
                            int copy, spmm_csr_t *out);
 
+/* More than 2^31 - 1 stored entries: 64-bit row offsets (rowptr[n_rows+1] as long long); colidx / vals as above.
+ * Not part of the reference's data model (its rowPtr is int32); every other call keeps its int32 meaning.
+ * Checks as the 32-bit entries: rowptr[0] == 0, rowptr[n_rows] == nnz, non-NULL arrays (else SPMM_ERR_INVALID); a row of
+ * more than 2^31 - 1 entries (possible only with duplicates) is SPMM_ERR_UNSUPPORTED. The rows are cut into segments of at
+ * most 2^30 non-zeros each (a longer row is a segment of its own), found on the device when the handle is created; each
+ * segment keeps a rebased int32 copy of its row pointer (4 bytes per row in all) and borrows its slices of colidx / vals.
+ * _device64 with copy=0 borrows the three arrays as spmm_csr_create_device does; a caller who changes the pattern must
+ * create the handle again.
+ * On such a handle (DESIGN.md section 4.8):
+ *   - every device multiply form runs the int32 kernels segment after segment on the caller's stream, and so do the host
+ *     forms built on them; AUTO decides per segment from that segment's schedule (merge-path, the stream kernel at k = 1
+ *     from stream.min_nnz non-zeros, else the row kernel) and never builds a tile layout;
+ *   - ROWS, MERGE and STREAM run on every segment (STREAM checks its shape per segment, before anything is launched, and
+ *     stays bit-identical to the reference); TILED and BSR are SPMM_ERR_UNSUPPORTED; other ids as on int32 handles;
+ *   - spmm_csr_build_tiles(_for_k), spmm_csr_build_bsr, spmm_csr_column_block, spmm_csr_device_ptrs and
+ *     spmm_csr_download are SPMM_ERR_UNSUPPORTED (the last two: use the 64-bit forms below);
+ *   - spmm_csr_info, spmm_csr_schedule (bins summed over the segments, global maximum and mean, auto_kernel merge-path if
+ *     any segment picked it), spmm_csr_column_span, spmm_nnz_range_rows, spmm_csr_update_values_host / _device and
+ *     spmm_csr_destroy work as on int32 handles. */
+int spmm_csr_create_host64(int device, int n_rows, int n_cols, long long nnz,
+                           const long long *rowptr, const int *colidx, const double *vals,
+                           spmm_csr_t *out);
+int spmm_csr_create_device64(int device, int n_rows, int n_cols, long long nnz,
+                             const long long *d_rowptr, const int *d_colidx, const double *d_vals,
+                             int copy, spmm_csr_t *out);
+/* The device arrays and the host copy of a handle with 64-bit row offsets (an int32 handle: SPMM_ERR_UNSUPPORTED). */
+int spmm_csr_device_ptrs64(spmm_csr_t A, const long long **d_rowptr, const int **d_colidx, const double **d_vals);
+int spmm_csr_download64(spmm_csr_t A, long long *rowptr, int *colidx, double *vals);
+
 /* a7: the CSR assembly of readMatrixMarketFile (utils.cpp:124-181) on the device.
  * Input = the file's coordinate records in file order, 0-based. Semantics reproduced
  * bit-exactly: symmetric!=0 mirrors off-diagonal records (:146-152), each row is ordered
@@ -303,7 +332,8 @@ int spmm_gen_fat_vector_device(int device, double *d_out, long long n_elems, lon
 /* Measurement knob (not needed for correct results): override the automatic team shape.
  * keys: rows.kl rows.nv rows.np rows.unroll rows.vec rows.ctas_per_sm rows.tile rows.prefetch merge.items merge.wave
  *       tiled tiled.thr tiled.chunk tiled.depth tiled.pool tiled.ns tiled.ksplit tiled.group tiled.stride tiled.pdl
- *       tiled.auto_after stream stream.tile stream.kmax stream.min_nnz host.slabs reset
+ *       tiled.auto_after stream stream.tile stream.kmax stream.min_nnz host.slabs seg.max_nnz reset
+ * seg.max_nnz: non-zeros per segment of the handles with 64-bit row offsets created after it is set (tests; default 2^30).
  * An unknown key fails with SPMM_ERR_INVALID. */
 int spmm_tune_set(const char *key, int value);
 

@@ -45,6 +45,10 @@ PROTOTYPES = {
     "spmm_device_info": (_i, [_i, _pi, _pll, _pll]),
     "spmm_csr_create_host": (_i, [_i, _i, _i, _ll, _p, _p, _p, C.POINTER(_p)]),
     "spmm_csr_create_device": (_i, [_i, _i, _i, _ll, _p, _p, _p, _i, C.POINTER(_p)]),
+    "spmm_csr_create_host64": (_i, [_i, _i, _i, _ll, _p, _p, _p, C.POINTER(_p)]),
+    "spmm_csr_create_device64": (_i, [_i, _i, _i, _ll, _p, _p, _p, _i, C.POINTER(_p)]),
+    "spmm_csr_device_ptrs64": (_i, [_p, C.POINTER(_p), C.POINTER(_p), C.POINTER(_p)]),
+    "spmm_csr_download64": (_i, [_p, _p, _p, _p]),
     "spmm_csr_from_coo_host": (_i, [_i, _i, _i, _ll, _p, _p, _p, _i, C.POINTER(_p)]),
     "spmm_csr_from_coo_device": (_i, [_i, _i, _i, _ll, _p, _p, _p, _i, C.POINTER(_p)]),
     "spmm_mm_read": (_i, [C.c_char_p, _pi, _pi, _pll, _pi, C.POINTER(_p), C.POINTER(_p), C.POINTER(_p)]),

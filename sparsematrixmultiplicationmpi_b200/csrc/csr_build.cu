@@ -396,6 +396,8 @@ int spmm_csr_from_coo_host(int device, int n_rows, int n_cols, long long n_entri
 int spmm_csr_column_block(spmm_csr_t A, int col_begin, int col_end, spmm_csr_t *out)
 {
     SPMM_REQUIRE(A != nullptr && out != nullptr, "handle is NULL");
+    if (A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_column_block", "spmm_csr_download64 and a handle built from the block's arrays");
     SPMM_REQUIRE(0 <= col_begin && col_begin <= col_end && col_end <= A->n_cols, "column range outside the matrix");
     SPMM_CUDA(cudaSetDevice(A->device));
     const int n_rows = A->n_rows;

@@ -288,6 +288,8 @@ using namespace spmm;
 extern "C" int spmm_csr_build_bsr(spmm_csr_t A, int block_dim, int *out_dim)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
+    if (A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_build_bsr", "SPMM_KERNEL_AUTO, ROWS, MERGE or STREAM");
     SPMM_REQUIRE(block_dim == -1 || block_dim == 0 || (block_dim >= 2 && block_dim <= 6),
                  "block_dim must be 0 (drop the view), 2..6, or -1 (largest that fits)");
     auto set = [&](int b) {

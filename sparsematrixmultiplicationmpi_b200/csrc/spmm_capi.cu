@@ -167,11 +167,11 @@ int build_schedule(spmm_csr_s *A, cudaStream_t stream)
     return SPMM_OK;
 }
 
-int make_handle(int device, int n_rows, int n_cols, long long nnz, spmm_csr_s **out)
+int make_handle(int device, int n_rows, int n_cols, long long nnz, spmm_csr_s **out, bool offsets64)
 {
     SPMM_REQUIRE(out != nullptr, "out handle is NULL");
     SPMM_REQUIRE(n_rows >= 0 && n_cols >= 0 && nnz >= 0, "negative size");
-    SPMM_REQUIRE(nnz <= 2147483647LL, "nnz exceeds the int32 rowPtr of the reference data model");
+    SPMM_REQUIRE(offsets64 || nnz <= 2147483647LL, "nnz exceeds the int32 rowPtr of the reference data model");
     int count = 0;
     SPMM_CUDA(cudaGetDeviceCount(&count));
     SPMM_REQUIRE(device >= 0 && device < count, "no such CUDA device");
@@ -257,6 +257,7 @@ int spmm_tune_set(const char *key, int value)
     else if (k == "rows.ctas_per_sm") t.rows_ctas_per_sm = value;
     else if (k == "merge.items") t.merge_items = value;
     else if (k == "merge.wave") t.merge_wave = value;
+    else if (k == "seg.max_nnz") t.seg_max_nnz = value;
     else if (k == "reset") t = Tuning();
     else
     {
@@ -347,9 +348,13 @@ int spmm_csr_destroy(spmm_csr_t A)
     if (A->owns)
     {
         cudaFree(A->d_rowptr);
+        cudaFree(A->d_rowptr64);
         cudaFree(A->d_colidx);
         cudaFree(A->d_vals);
     }
+    for (spmm_csr_s *S : A->segs)
+        spmm_csr_destroy(S);
+    cudaFree(A->d_seg_rowptr);
     free_tiles(A);
     drop_bounds(A, -1);
     cudaFree(A->d_B);
@@ -384,6 +389,8 @@ int spmm_csr_info(spmm_csr_t A, int *n_rows, int *n_cols, long long *nnz, int *d
 int spmm_csr_device_ptrs(spmm_csr_t A, const int **d_rowptr, const int **d_colidx, const double **d_vals)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
+    if (A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_device_ptrs", "spmm_csr_device_ptrs64");
     if (d_rowptr) *d_rowptr = A->d_rowptr;
     if (d_colidx) *d_colidx = A->d_colidx;
     if (d_vals) *d_vals = A->d_vals;
@@ -405,6 +412,8 @@ int spmm_csr_update_values_device(spmm_csr_t A, const double *d_vals, void *stre
 int spmm_csr_download(spmm_csr_t A, int *rowptr, int *colidx, double *vals)
 {
     SPMM_REQUIRE(A != nullptr, "handle is NULL");
+    if (A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_download", "spmm_csr_download64");
     SPMM_CUDA(cudaSetDevice(A->device));
     if (rowptr)
         SPMM_CUDA(cudaMemcpy(rowptr, A->d_rowptr, sizeof(int) * ((size_t)A->n_rows + 1), cudaMemcpyDeviceToHost));
@@ -543,6 +552,8 @@ int spmm_nnz_range_rows(spmm_csr_t A, long long nnz_begin, long long nnz_end, in
         return SPMM_OK;
     }
     SPMM_CUDA(cudaSetDevice(A->device));
+    if (A->d_rowptr64)
+        return nnz_range_rows64(A, nnz_begin, nnz_end, first_row, last_row);
     int *d_out = nullptr;
     SPMM_CUDA(cudaMalloc(&d_out, 2 * sizeof(int)));
     nnz_range_rows_kernel<<<1, 1>>>(A->d_rowptr, A->n_rows, (int)nnz_begin, (int)nnz_end, d_out);

@@ -147,15 +147,52 @@ static int auto_kernel(spmm_csr_s *A, const Request &r)
     return tiled_auto_ok(A, r) ? SPMM_KERNEL_TILED : SPMM_KERNEL_ROWS;
 }
 
+static const char *const STREAM_SHAPE_MSG =
+    "stream kernel: k must be 1, 2, 4 or 8 (B 16-byte aligned with an even leading dimension from k = 2), rows of at most 3072 / k non-zeros";
+
+// A handle with 64-bit row offsets: the request in each segment's own rows and non-zeros, segment after segment on `stream`.
+// A row lies in one segment, so partial rows of a non-zero range keep their meaning; AUTO decides per segment. Nothing is
+// launched unless every segment can serve an explicit STREAM request.
+static int multiply_segments(spmm_csr_s *A, const Request &r, int kernel, cudaStream_t stream)
+{
+    if (kernel == SPMM_KERNEL_TILED || kernel == SPMM_KERNEL_BSR)
+    {
+        set_error("the tiled and BSR kernels need a layout that is not built for handles with 64-bit row offsets");
+        return SPMM_ERR_UNSUPPORTED;
+    }
+    std::vector<std::pair<spmm_csr_s *, Request>> parts;
+    for (spmm_csr_s *S : A->segs)
+    {
+        const int r0 = std::max(r.row_begin, S->seg_row0), r1 = std::min(r.row_end, S->seg_row0 + S->n_rows);
+        if (r0 >= r1)
+            continue;
+        Request q = r;
+        q.row_begin = r0 - S->seg_row0;
+        q.row_end = r1 - S->seg_row0;
+        q.nnz_lo = std::clamp(r.nnz_lo - S->seg_nnz0, 0LL, S->nnz);
+        q.nnz_hi = std::clamp(r.nnz_hi - S->seg_nnz0, q.nnz_lo, S->nnz);
+        q.c_row0 = q.row_begin;
+        q.C = r.C + (long long)(r0 - r.c_row0) * r.ldc;
+        if (kernel == SPMM_KERNEL_STREAM)
+            SPMM_REQUIRE(stream_shape_ok(S, q.B, q.ldb, q.C, q.ldc, q.kc), STREAM_SHAPE_MSG);
+        parts.emplace_back(S, q);
+    }
+    for (const auto &[S, q] : parts)
+        if (int rc = multiply(S, q, kernel, stream))
+            return rc;
+    return SPMM_OK;
+}
+
 int multiply(spmm_csr_s *A, const Request &r, int kernel, cudaStream_t stream)
 {
     SPMM_CUDA(cudaSetDevice(A->device));
+    if (A->d_rowptr64)
+        return multiply_segments(A, r, kernel, stream);
     // what an explicit request needs from the handle is checked at launch time
     if (kernel == SPMM_KERNEL_BSR)
         SPMM_REQUIRE(A->bsr_b != 0, "BSR kernel requested but spmm_csr_build_bsr was not called (or found no block size)");
     if (kernel == SPMM_KERNEL_STREAM)
-        SPMM_REQUIRE(stream_shape_ok(A, r.B, r.ldb, r.C, r.ldc, r.kc),
-                     "stream kernel: k must be 1, 2, 4 or 8 (B 16-byte aligned with an even leading dimension from k = 2), rows of at most 3072 / k non-zeros");
+        SPMM_REQUIRE(stream_shape_ok(A, r.B, r.ldb, r.C, r.ldc, r.kc), STREAM_SHAPE_MSG);
     if (kernel == SPMM_KERNEL_TILED)
         if (int rc = tiled_check(A, r))
             return rc;

@@ -75,6 +75,7 @@ struct Tuning
     int stream_auto_kmax = 1; // AUTO takes the stream kernel up to this k ...
     int stream_auto_min_nnz = 4 << 20; // ... from this many non-zeros (measured: equal to the row kernel at 2.6 M non-zeros, 43 against 56 us at 10.5 M; profiles/r1_stream.md)
     int stream_tile = 0;    // stream kernel: non-zeros per tile (0 = 4096 / k)
+    int seg_max_nnz = 1 << 30; // 64-bit handles: non-zeros per segment (a longer row is a segment of its own); read at creation
 };
 Tuning &tuning();
 
@@ -128,6 +129,13 @@ struct spmm_csr_s
     size_t carry_elems = 0, carry_rows = 0;
     cudaEvent_t carry_done = nullptr;
     cudaStream_t carry_stream = nullptr; // stream of the last merge launch (carry_done was recorded there)
+    // 64-bit row offsets (spmm_csr64.cu): d_rowptr stays nullptr; the rows are cut into segments, ordinary handles that
+    // borrow their slices of d_colidx / d_vals and own nothing but their place in d_seg_rowptr (rebased int32 row pointers)
+    long long *d_rowptr64 = nullptr;
+    std::vector<spmm_csr_s *> segs;
+    int *d_seg_rowptr = nullptr;
+    int seg_row0 = 0;       // on a segment: its first row and first non-zero in the 64-bit handle
+    long long seg_nnz0 = 0;
 };
 
 namespace spmm
@@ -182,8 +190,11 @@ int launch_stream(const spmm_csr_s *A, const double *d_B, long long ldb, double 
 int cached_bounds(const spmm_csr_s *A, int kind, int grid, cudaStream_t stream, const int **out,
                   const std::function<void(int *)> &fill);
 void drop_bounds(spmm_csr_s *A, int kind); // kind < 0: all
-// handle plumbing shared by spmm_capi.cu and csr_build.cu
-int make_handle(int device, int n_rows, int n_cols, long long nnz, spmm_csr_s **out);
+// handle plumbing shared by spmm_capi.cu, csr_build.cu and spmm_csr64.cu; offsets64: nnz may exceed 2^31 - 1
+int make_handle(int device, int n_rows, int n_cols, long long nnz, spmm_csr_s **out, bool offsets64 = false);
 int alloc_arrays(spmm_csr_s *A);
 int build_schedule(spmm_csr_s *A, cudaStream_t stream);
+// 64-bit handles (spmm_csr64.cu): SPMM_ERR_UNSUPPORTED for a call that needs int32 row offsets, naming what to use instead
+int refuse_offsets64(const char *call, const char *instead);
+int nnz_range_rows64(const spmm_csr_s *A, long long nnz_begin, long long nnz_end, int *first_row, int *last_row);
 } // namespace spmm

@@ -1671,11 +1671,18 @@ using namespace spmm;
 extern "C"
 {
 
-int spmm_csr_build_tiles(spmm_csr_t A, int rows_per_tile, int box_rows) { return build_tiles(A, rows_per_tile, box_rows, 0, 0); }
+int spmm_csr_build_tiles(spmm_csr_t A, int rows_per_tile, int box_rows)
+{
+    if (A && A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_build_tiles", "SPMM_KERNEL_AUTO, ROWS, MERGE or STREAM");
+    return build_tiles(A, rows_per_tile, box_rows, 0, 0);
+}
 
 int spmm_csr_build_tiles_for_k(spmm_csr_t A, int rows_per_tile, int box_rows, int k)
 {
     SPMM_REQUIRE(k >= 0, "k is negative");
+    if (A && A->d_rowptr64)
+        return refuse_offsets64("spmm_csr_build_tiles_for_k", "SPMM_KERNEL_AUTO, ROWS, MERGE or STREAM");
     if (k == 0)
         return build_tiles(A, rows_per_tile, box_rows, 0, 0);
     return build_tiles(A, rows_per_tile, box_rows, tiles_kt_for(k), tiles_ksplit_for(k));

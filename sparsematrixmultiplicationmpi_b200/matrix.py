@@ -75,6 +75,42 @@ class DeviceCSR:
         return cls(h.value)
 
     @classmethod
+    def from_csr64(cls, rowptr, colidx, vals, n_rows: int, n_cols: int, device: int = 0, copy: bool = True) -> "DeviceCSR":
+        """A CSR with 64-bit row offsets, for more than 2^31 - 1 stored entries (spmm_csr_create_host64 / _device64):
+        rowptr int64[n_rows+1], colidx int32[nnz], vals float64[nnz]. C-contiguous numpy arrays are uploaded (copy is
+        ignored); contiguous CUDA tensors on cuda:`device` are copied, or borrowed with copy=False (the DeviceCSR then
+        keeps them alive; changing the pattern needs a new handle). The handle runs the int32 kernels on segments of rows
+        (include/spmm_b200.h lists what it supports); every method works on it or raises SpmmError."""
+        arrays = (rowptr, colidx, vals)
+        if all(isinstance(a, np.ndarray) for a in arrays):
+            ok_dtypes = [a.dtype for a in arrays] == [np.int64, np.int32, np.float64]
+            ok_layout = all(a.ndim == 1 and a.flags.c_contiguous for a in arrays)
+            sizes = [a.size for a in arrays]
+            host = True
+        else:
+            import torch
+            if not all(isinstance(a, torch.Tensor) and a.is_cuda and a.device.index == device for a in arrays):
+                raise ValueError(f"rowptr/colidx/vals must be three numpy arrays or three CUDA tensors on cuda:{device}")
+            ok_dtypes = [a.dtype for a in arrays] == [torch.int64, torch.int32, torch.float64]
+            ok_layout = all(a.dim() == 1 and a.is_contiguous() for a in arrays)
+            sizes = [a.numel() for a in arrays]
+            host = False
+        if not (ok_dtypes and ok_layout):
+            raise ValueError("rowptr, colidx, vals must be contiguous 1-D int64, int32 and float64 arrays")
+        if sizes[0] != n_rows + 1 or sizes[1] != sizes[2]:
+            raise ValueError(f"rowptr must hold n_rows+1 = {n_rows + 1} offsets and colidx / vals the same count")
+        nnz = sizes[1]
+        h = C.c_void_p()
+        if host:
+            _cabi.check(_cabi.lib().spmm_csr_create_host64(device, n_rows, n_cols, nnz, rowptr.ctypes.data,
+                                                           colidx.ctypes.data, vals.ctypes.data, C.byref(h)))
+            return cls(h.value)
+        _cabi.check(_cabi.lib().spmm_csr_create_device64(device, n_rows, n_cols, nnz, C.c_void_p(rowptr.data_ptr()),
+                                                         C.c_void_p(colidx.data_ptr()), C.c_void_p(vals.data_ptr()),
+                                                         int(bool(copy)), C.byref(h)))
+        return cls(h.value, owner=None if copy else arrays)
+
+    @classmethod
     def from_coo_host(cls, n_rows, n_cols, rows, cols, vals, symmetric=False, device: int = 0) -> "DeviceCSR":
         """The CSR assembly of readMatrixMarketFile (utils.cpp:124-181) done on the device."""
         rows = np.ascontiguousarray(rows, dtype=np.int32)
@@ -121,6 +157,15 @@ class DeviceCSR:
         _cabi.check(_cabi.lib().spmm_csr_download(self.handle, rowptr.ctypes.data, colidx.ctypes.data,
                                                   vals.ctypes.data))
         return SparseMatrix(vals, colidx, rowptr, self.n_rows, self.n_cols)
+
+    def download64(self) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(rowptr int64, colidx int32, vals float64) of a handle with 64-bit row offsets (spmm_csr_download64)."""
+        rowptr = np.empty(self.n_rows + 1, dtype=np.int64)
+        colidx = np.empty(self.nnz, dtype=np.int32)
+        vals = np.empty(self.nnz, dtype=np.float64)
+        _cabi.check(_cabi.lib().spmm_csr_download64(self.handle, rowptr.ctypes.data, colidx.ctypes.data,
+                                                    vals.ctypes.data))
+        return rowptr, colidx, vals
 
     def schedule(self) -> dict:
         bins = (C.c_longlong * 8)()
